@@ -3,6 +3,8 @@
 synthetic 1x1x96x112x96 skeleton volumes (BASELINE.json configs[1]; configs[3] under torchrun with N ranks).
 
   python bench.py --gpus 1 --steps K --warmup W            our arm (hand-written sm_100a kernels)
+      ... --dump-outputs DIR                               also writes the last timed step's loss and updated
+                                                            parameters as DIR/*.npy (see dump_outputs)
   python bench.py --impl reference --steps K --warmup W     the reference's CPU path (oracle port, host cores), on the
                                                             SAME full 96x112x96 volume
   torchrun ... bench.py --gpus N ...                        data parallel over subjects, one rank per GPU
@@ -304,6 +306,25 @@ def _quiet():
     return contextlib.redirect_stdout(io.StringIO())
 
 
+DUMP_SAMPLE = 1 << 20     # elements kept of a larger tensor: the 44 fp32 parameters alone are 65 MB
+
+
+def dump_outputs(out_dir, loss, model):
+    """--dump-outputs: what the last timed step hands its caller, as out_dir/<name>.npy (float32): `loss` = the
+    (mean, sum) the step returns, and `param.<name>` = every parameter as the step's SGD update left it.  A tensor of
+    more than DUMP_SAMPLE elements is flattened and sampled at DUMP_SAMPLE positions drawn by a fixed-seed generator,
+    the same positions on every run, so that the dumps of two builds compare element for element (about 31 MB)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = [("loss", loss)] + [("param." + n, p) for n, p in model.named_parameters()]
+    for name, t in arrays:
+        a = t.detach().float().cpu().numpy()
+        if a.size > DUMP_SAMPLE:
+            pick = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.reshape(-1)[pick]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -345,8 +366,11 @@ def run_ours(args):
     # gradient bucket with the NCCL all-reduces enqueued eagerly in between (NCCL itself is never captured)
     trainer.use_cuda_graph = not args.no_cuda_graph
 
+    last_loss = [None]
+
     def step_resident(i):
-        return trainer.train_step_device(xs_d[i % n_data], ls_d[i % n_data], opt, reducer)
+        last_loss[0] = trainer.train_step_device(xs_d[i % n_data], ls_d[i % n_data], opt, reducer)
+        return last_loss[0]
 
     def sync_all():
         torch.cuda.synchronize()
@@ -396,6 +420,8 @@ def run_ours(args):
     launches = int(round(launches_per_step * args.steps))
     clocks = sampler.stop()
     value = world * args.steps / secs
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_loss[0], model)
 
     # roofline of the dominant kernels: 26 launches / step, fprop + dgrad of the 13 Cin >= 32 convs (implicit GEMM on
     # tcgen05: conv3d_igemm_kernel, and conv3d_slab_kernel for the Cout <= 64 layers)
@@ -723,7 +749,13 @@ def main():
     ap.add_argument("--no-torch-gpu", action="store_true")
     ap.add_argument("--no-cuda-graph", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="profiling runs only: skip the learning() leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's loss and updated parameters to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.inference or args.sweep):
+        ap.error("--dump-outputs applies to the training benchmark of our arm only")
     if args.impl == "reference":
         return run_reference_arm(args)
     if args.inference:

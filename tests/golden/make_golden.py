@@ -1,6 +1,6 @@
-"""Regenerates the fixtures under tests/golden/.  Run in the build container (needs /root/reference):
+"""Regenerates the fixtures under tests/golden/.  Needs a checkout of the reference (see tests/harness.py):
 
-    python tests/golden/make_golden.py
+    UNETSULC_REFERENCE=<checkout> python tests/golden/make_golden.py
 
 Fixtures (small, committed):
   plateau_traces.json ........ decisions of the REFERENCE's own DivideLr / FineTunning (divide_lr.py, fine_tunning.py)
@@ -146,7 +146,7 @@ def esi_cases():
 
 
 if __name__ == "__main__":
-    assert harness.reference_available(), "needs /root/reference"
+    assert harness.reference_available(), "set UNETSULC_REFERENCE to a checkout of the reference"
     json.dump(plateau_traces(), open(os.path.join(HERE, "plateau_traces.json"), "w"))
     np.savez_compressed(os.path.join(HERE, "dataset_cases.npz"), **dataset_cases())
     json.dump(reference_training(), open(os.path.join(HERE, "reference_training.json"), "w"), indent=1)

@@ -1,6 +1,7 @@
-"""Boundary harness: runs the reference's UNMODIFIED host code (/root/reference/{training,pattern_class,dataset,
-divide_lr}.py) with `deepsulci.*` / `soma` / `sigraph` injected through sys.modules (unetsulc_b200.deepsulci_shim).
-Only usable where /root/reference exists (this container); the GPU box uses the fixtures under tests/golden/.
+"""Boundary harness: runs the reference's UNMODIFIED host code ({training,pattern_class,dataset,divide_lr}.py of a
+checkout of github.com/neurospin-projects/2022_pauriau_unetsulc) with `deepsulci.*` / `soma` / `sigraph` injected
+through sys.modules (unetsulc_b200.deepsulci_shim).  The checkout is not part of this repository: set
+UNETSULC_REFERENCE to its directory to use it.  Without it the tests use the fixtures under tests/golden/.
 """
 import contextlib
 import importlib
@@ -12,14 +13,14 @@ import sys
 import numpy as np
 import torch
 
-REF = "/root/reference"
+REF = os.environ.get("UNETSULC_REFERENCE", "")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 
 def reference_available():
-    return os.path.isdir(REF)
+    return bool(REF) and os.path.isdir(REF)
 
 
 def synthetic_cohort(n_subjects=3, shape=(16, 16, 16), n_classes=6, seed=0):

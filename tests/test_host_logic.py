@@ -166,9 +166,9 @@ def test_shard_subjects():
 
 def test_reference_host_code_runs_unmodified_on_the_boundary(tmp_path):
     """The reference's own training.py (unmodified) driven through the deepsulci import boundary with the oracle:
-    must reproduce the committed trace (skipped where /root/reference is absent, e.g. on the GPU box)."""
+    must reproduce the committed trace (skipped unless UNETSULC_REFERENCE names a checkout of the reference)."""
     if not harness.reference_available():
-        pytest.skip("/root/reference not present")
+        pytest.skip("no checkout of the reference: set UNETSULC_REFERENCE")
     from oracle.unet3d_ref import UNet3DRef
     method = harness.run_reference_training(str(tmp_path), UNet3DRef, n_epochs=2,
                                             patience={'divide_lr': 1, 'early_stopping': 3})
