@@ -542,6 +542,15 @@ def test_upsample_concat_fwd_bwd(din, dout):
         dx = ops.upcat_bwd(ops.ActView(to_ndhwc(dcat), N, *dout, C, ld=Cs + C, coff=Cs), *din, separable=separable)
         torch.cuda.synchronize()
         assert rel_l2(from_view(dx), x.grad) < 4e-3, separable
+    # with the fused GroupNorm-backward statistics (two-pass kernels on the non-2x ratios): same dx, accumulators ==
+    # fp64 sums of the stored tensor within the fixed-point bound (tests/test_gpu_step_oracle.py)
+    from tests.test_gpu_step_oracle import Oracle, spy_upcat_bwd
+    orc = Oracle()
+    r = ops.ActView(to_ndhwc(bf16_round(torch.randn(N, C, *din, device="cuda", generator=g).relu())), N, *din, C)
+    dx2, _ = spy_upcat_bwd(ops.upcat_bwd, orc, ops.ActView(to_ndhwc(dcat), N, *dout, C, ld=Cs + C, coff=Cs), *din,
+                           stat_r=r)
+    assert torch.equal(dx2.buf, dx.buf)
+    assert all(v <= 1.0 for v in orc.worst.values()), orc.worst
 
 
 @pytest.mark.parametrize("N,C,din", [(1, 64, (5, 6, 9)), (1, 128, (24, 28, 24)), (2, 256, (3, 5, 4)), (1, 512, (6, 7, 6))])
@@ -701,6 +710,181 @@ def test_sgd_matches_torch():
     torch.cuda.synchronize()
     for p, rp in zip(ps, ref_ps):
         assert torch.allclose(p, rp.detach(), rtol=1e-6, atol=1e-7)
+
+
+def test_sgd_multi_launch_odd_views_and_grad_scale():
+    """> 64 tensors (two launches of sgd_multi_kernel), numels that are not multiples of 4, parameters that are views
+    at odd float offsets of one flat buffer (as the data-parallel buckets are: the scalar path), grad_scale != 1.
+    Against the fp64 recurrence v <- mu v + s g, p <- p - lr v with lr, mu, s rounded to fp32 as the kernel receives
+    them.  Bound per element after k steps: 5 k u P, P = |p0| + sum_j lr Av_j, Av_j = mu Av_(j-1) + |s g_j|: step j
+    adds at most 3 u Av_j to the error of v (mu v, s g, their sum), the error of v carries through mu, so
+    e_v(j) <= 3 j u Av_j, and p takes lr e_v(j) plus 2 u (|p| + lr |v|) per step: e_p(k) <= 3 k u P + 2 k u P."""
+    ops = _ops()
+    g = torch.Generator(device="cuda").manual_seed(13)
+    numels = [(i * 37) % 301 + 1 for i in range(70)] + [4099, 8192 + 3, 4096]
+    flat = torch.randn(sum(numels) + len(numels), device="cuda", generator=g)
+    ps, off = [], 1
+    for n in numels:                       # every view starts one float after the end of the previous one
+        ps.append(flat[off:off + n])
+        off += n + 1
+    moms = [torch.zeros_like(p) for p in ps]
+    lr, mu, s, steps = 1e-2, 0.9, 0.37, 3
+    lr32, mu32, s32 = (float(torch.tensor(c, dtype=torch.float32)) for c in (lr, mu, s))
+    p64 = [p.double().clone() for p in ps]
+    v64 = [torch.zeros_like(q) for q in p64]
+    P = [q.abs() for q in p64]
+    Vabs = [torch.zeros_like(q) for q in p64]
+    for _ in range(steps):
+        grads = [torch.randn(n, device="cuda", generator=g) for n in numels]
+        ops.sgd_step(ps, grads, moms, lr, mu, grad_scale=s)
+        for i, gr in enumerate(grads):
+            v64[i] = mu32 * v64[i] + s32 * gr.double()
+            p64[i] = p64[i] - lr32 * v64[i]
+            Vabs[i] = mu32 * Vabs[i] + abs(s32) * gr.double().abs()
+            P[i] = P[i] + lr32 * Vabs[i]
+    torch.cuda.synchronize()
+    u = 2.0 ** -24
+    for i, (p, ref, mag) in enumerate(zip(ps, p64, P)):
+        err = (p.double() - ref).abs()
+        assert bool((err <= 5 * steps * u * mag + 1e-30).all()), (i, numels[i], float(err.max()))
+
+
+def test_pack_conv_weights_multi_many_layers():
+    """> 16 layers (several launches, kMaxPackLayers): every trunk (cout, cin) and Cin in {384, 768}; bit-equal to
+    pack_conv_weights and to the bf16 permutation of the fp32 master (Wf[tap][co][ci], Wd[26 - tap][ci][co])."""
+    ops = _ops()
+    g = torch.Generator(device="cuda").manual_seed(14)
+    trunk = [(64, 32), (64, 64), (128, 64), (128, 128), (256, 128), (256, 256), (512, 256), (256, 768), (256, 256),
+             (128, 384), (128, 128), (64, 192), (64, 64)]
+    shapes = trunk + trunk[::-1] + [(64, 384), (128, 768), (512, 512)]
+    ws = [torch.randn(co, ci, 3, 3, 3, device="cuda", generator=g) * 0.05 for co, ci in shapes]
+    outs = ops.pack_conv_weights_multi(ws)
+    torch.cuda.synchronize()
+    assert len(outs) == len(ws)
+    for (co, ci), w, (wf, wd) in zip(shapes, ws, outs):
+        wb = w.to(torch.bfloat16)
+        assert torch.equal(wf, wb.permute(2, 3, 4, 0, 1).reshape(27, co, ci)), (co, ci)
+        assert torch.equal(wd, wb.flip(2, 3, 4).permute(2, 3, 4, 1, 0).reshape(27, ci, co)), (co, ci)
+        wf1, wd1 = ops.pack_conv_weights(w)
+        assert torch.equal(wf, wf1) and torch.equal(wd, wd1), (co, ci)
+
+
+BSTATS_CASES = [
+    ("dgrad", (64, 64, 8, 12, 64)), ("dgrad", (128, 64, 6, 8, 32)), ("dgrad", (256, 128, 6, 7, 6)),
+    ("pool", (64, 8, 10, 12)), ("pool", (128, 7, 9, 11)), ("pool", (256, 6, 6, 8)),
+    ("up", (64, (5, 6, 9), (10, 12, 18))), ("up", (128, (24, 28, 24), (48, 56, 48))), ("up", (512, (6, 7, 6), (12, 14, 12))),
+    ("up", (128, (8, 13, 10), (17, 26, 21))), ("up", (256, (4, 6, 5), (8, 13, 10))), ("up", (512, (2, 3, 2), (4, 6, 5))),
+]
+
+
+@pytest.mark.parametrize("scale", [1.0, 1e-4, 1e-6])
+@pytest.mark.parametrize("case", BSTATS_CASES, ids=lambda c: "%s-%s" % (c[0], "x".join(str(v) for v in c[1][:2])))
+def test_bstats_producers_at_gradient_scale(case, scale):
+    """The kernels that produce a gradient at a GroupNorm output and accumulate its backward statistics (dgrad
+    epilogue, pooling adjoint, upsample adjoint: single-pass 2x and two-pass non-2x), with the gradient scaled to the
+    magnitudes of a real step (mean cross-entropy over ~2e4 voxels: 1e-5 .. 1e-6 per voxel).  Each output against fp64,
+    the accumulators against fp64 sums of the stored tensor with the fixed-point bound, and dr / dgamma / dbeta of the
+    accumulator route against the closed-form fp64 GroupNorm backward, relative to the sum of |terms| per channel
+    (bounds: tests/test_gpu_step_oracle.py)."""
+    ops = _ops()
+    from tests.test_gpu_step_oracle import (Oracle, spy_conv3d_dgrad_gn_bstats, spy_maxpool3d_bwd_add,
+                                            spy_relu_gn_bwd_from_stats, spy_upcat_bwd)
+    kind, shp = case
+    G = 32
+    orc = Oracle()
+    g = torch.Generator(device="cuda").manual_seed(71)
+
+    def act(C, dims, s=1.0, relu=False):
+        t = torch.randn(1, *dims, C, device="cuda", generator=g) * s
+        return ops.ActView((t.relu() if relu else t).to(torch.bfloat16), 1, *dims, C)
+
+    if kind == "dgrad":
+        Cdy, Cdx, D, H, W = shp
+        dims, C = (D, H, W), Cdx
+        w = torch.randn(Cdy, Cdx, 3, 3, 3, device="cuda", generator=g) * (1.0 / (27 * Cdy) ** 0.5)
+        _, wd = ops.pack_conv_weights(w)
+        r = act(C, dims, relu=True)
+        dx = ops.ActView.alloc(1, D, H, W, C, "cuda")
+        acc = spy_conv3d_dgrad_gn_bstats(ops.conv3d_dgrad_gn_bstats, orc, act(Cdy, dims, scale), wd, dx, Cdy, Cdx, r)
+    elif kind == "pool":
+        C, D, H, W = shp
+        dims = (D, H, W)
+        r = act(C, dims, relu=True)
+        dx, acc = spy_maxpool3d_bwd_add(ops.maxpool3d_bwd_add, orc, act(C, dims), act(C, dims, scale),
+                                        act(C, (D // 2, H // 2, W // 2), scale), stat_r=r)
+    else:
+        C, din, dout = shp
+        dims = din
+        r = act(C, din, relu=True)
+        dx, acc = spy_upcat_bwd(ops.upcat_bwd, orc, act(C, dout, scale), *din, stat_r=r)
+    gamma = torch.randn(C, device="cuda", generator=g) * 0.5 + 1.0
+    beta = torch.randn(C, device="cuda", generator=g) * 0.1
+    mr, _ = ops.relu_gn_stats(r, G, 1e-5, gamma, beta)
+    spy_relu_gn_bwd_from_stats(ops.relu_gn_bwd_from_stats, orc, acc, dx, r, G, gamma, mr)
+    print("%s scale %g: %s" % (case, scale, " ".join("%s=%.2e" % kv for kv in sorted(orc.worst.items()))))
+    assert all(v <= 1.0 for v in orc.worst.values()), orc.worst
+
+
+def _head_ce_bstats_call(ops, xv, labels, Wt, b, r, dx, xss):
+    """b2_head_ce_bstats with skip_dx_memset = 1 into the caller's dX buffer (ops.head_ce allocates its own)"""
+    lib = ops._lib.load()
+    N, Cin = xv.N, xv.C
+    Cout = Wt.shape[0]
+    dev = xv.buf.device
+    loss = torch.empty(2, dtype=torch.float32, device=dev)
+    count = torch.empty(1, dtype=torch.int32, device=dev)
+    preds = torch.full((N, xv.D, xv.H, xv.W), -1, dtype=torch.int32, device=dev)
+    dW = torch.empty(Cout, Cin, dtype=torch.float32, device=dev)
+    db = torch.empty(Cout, dtype=torch.float32, device=dev)
+    acc = torch.zeros(4 * Cin, dtype=torch.int64, device=dev)
+    ws = ops.Workspace.get(lib.b2_head_workspace_bytes(Cin), dev, "head")
+    Wc = Wt.reshape(Cout, Cin).contiguous()
+    ops._lib.check(lib.b2_head_ce_bstats(ops._p(xv.buf), ops._p(labels), N * xv.V, ops._p(Wc), ops._p(b), Cin, Cout,
+                                         1.0, ops._p(None), ops._p(preds), ops._p(dx.buf), ops._p(dW), ops._p(db),
+                                         ops._p(loss), ops._p(count), ops._p(ws), ws.numel(), ops._p(r.buf),
+                                         ops._p(acc), ops._p(xss), 1, ops._s()), "b2_head_ce_bstats")
+    return dict(loss=loss, count=count, preds=preds, dx=dx, dW=dW, db=db, dx_stats=acc)
+
+
+@pytest.mark.parametrize("Cout", [3, 56, 64])
+@pytest.mark.parametrize("deferred_apply", [False, True])
+@pytest.mark.parametrize("frac", [0.2, 0.0])
+def test_head_sparse_dx_rows_never_read(Cout, deferred_apply, frac):
+    """b2_head_ce_bstats with skip_dx_memset = 1 writes only the labelled rows of dX (the buffer is pre-filled with bf16
+    NaN here); relu_gn_bwd_from_stats(dy_row_labels=labels) must read the other rows as zero: dr, dgamma, dbeta finite
+    and equal to the fp64 reference with those rows zero.  frac = 0: no labelled voxel -> NaN loss, zero accumulators,
+    zero dr."""
+    ops = _ops()
+    from tests.test_gpu_step_oracle import Oracle, _block_count_max, _gn_bwd_check, head_check
+    x, Wt, b, labels = _head_inputs(19, D=9, H=11, W=13, Cout=Cout, frac=frac)
+    if frac == 0.0:
+        labels = torch.full_like(labels, -1)
+    N, Cin, D, H, W = x.shape
+    g = torch.Generator(device="cuda").manual_seed(20)
+    r = ops.ActView(to_ndhwc(x.relu()), N, D, H, W, Cin)
+    gamma = torch.randn(Cin, device="cuda", generator=g) * 0.5 + 1.0
+    beta = torch.randn(Cin, device="cuda", generator=g) * 0.2
+    mr, ss = ops.relu_gn_stats(r, 32, 1e-5, gamma, beta)
+    if deferred_apply:
+        xv, xss = r, ss
+    else:
+        xv = ops.ActView.alloc(N, D, H, W, Cin, "cuda")
+        ops.relu_gn_apply(r, ss, xv)
+        xss = None
+    dx = ops.ActView(torch.full((N, D, H, W, Cin), float("nan"), device="cuda", dtype=torch.bfloat16), N, D, H, W, Cin)
+    out = _head_ce_bstats_call(ops, xv, labels, Wt, b, r, dx, xss)
+    dr, dg, db = ops.relu_gn_bwd_from_stats(out["dx_stats"], dx, r, 32, gamma, mr, dy_row_labels=labels)
+    torch.cuda.synchronize()
+    assert bool(torch.isfinite(dr.buf.float()).all()) and bool(torch.isfinite(dg).all() and torch.isfinite(db).all())
+    orc = Oracle()
+    head_check(orc, xv, labels, Wt, b, out, True, 1.0, r, xss, True)
+    _gn_bwd_check(orc, "gn_bwd", dx, r, 32, gamma, mr, dr, dg, db, _block_count_max(labels, N * D * H * W) + 6, 296,
+                  labels)
+    assert all(v <= 1.0 for v in orc.worst.values()), orc.worst
+    if frac == 0.0:
+        assert bool(torch.isnan(out["loss"][0])) and int(out["count"]) == 0
+        assert int(out["dx_stats"].abs().sum()) == 0
+        assert float(dr.buf.float().abs().sum()) == 0.0 and float(dg.abs().sum()) == 0.0
 
 
 def test_fold_vote_bit_exact_vs_oracle():
