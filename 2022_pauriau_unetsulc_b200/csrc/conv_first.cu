@@ -12,7 +12,8 @@ namespace b2 {
 // round-1 kernel walked the taps one dependent L1 load at a time and was latency-bound at 680 GB/s); a tap is skipped
 // when no lane of the warp has a non-zero input there.  When stat_acc != NULL the kernel also accumulates, per
 // channel, sum and sum of squares of the STORED (ReLU'd, bf16-rounded) outputs — the GroupNorm statistics — into
-// the exact [COUT][4] accumulators of common.h (one atomic add per block and channel).
+// the exact [COUT][4] accumulators of common.h (one atomic add per block and channel).  COUT = 16 (32-filter networks)
+// sums one half-empty 32-column chunk: lanes 16..31 carry zeros and are not stored.
 template <int COUT>
 __global__ void __launch_bounds__(128)
 conv_first_fwd_kernel(const float* __restrict__ x, const float* __restrict__ w /*[COUT][27]*/,
@@ -25,9 +26,10 @@ conv_first_fwd_kernel(const float* __restrict__ x, const float* __restrict__ w /
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const long long V = (long long)N * D * H * W;
-  float st_s[COUT / 32], st_q[COUT / 32];   // lane L: channel 32*k + L, summed over this warp's voxels
+  constexpr int kChunks = (COUT + 31) / 32;
+  float st_s[kChunks], st_q[kChunks];   // lane L: channel 32*k + L, summed over this warp's voxels
 #pragma unroll
-  for (int k = 0; k < COUT / 32; ++k) { st_s[k] = 0.f; st_q[k] = 0.f; }
+  for (int k = 0; k < kChunks; ++k) { st_s[k] = 0.f; st_q[k] = 0.f; }
   for (long long v0 = ((long long)blockIdx.x * 4 + warp) * 32; v0 < V; v0 += (long long)gridDim.x * 128) {
     const long long v = v0 + lane;
     const bool active = v < V;
@@ -81,11 +83,11 @@ conv_first_fwd_kernel(const float* __restrict__ x, const float* __restrict__ w /
     }
     if (stat_acc != nullptr) {
 #pragma unroll
-      for (int k = 0; k < COUT / 32; ++k) {
+      for (int k = 0; k < kChunks; ++k) {
         float xs[32], xq[32];
 #pragma unroll
         for (int e = 0; e < 32; ++e) {
-          const float f = active ? __bfloat162float(__float2bfloat16_rn(acc[32 * k + e])) : 0.f;
+          const float f = (active && 32 * k + e < COUT) ? __bfloat162float(__float2bfloat16_rn(acc[32 * k + e])) : 0.f;
           xs[e] = f;
           xq[e] = f * f;
         }
@@ -98,7 +100,8 @@ conv_first_fwd_kernel(const float* __restrict__ x, const float* __restrict__ w /
   }
   if (stat_acc != nullptr) {
 #pragma unroll
-    for (int k = 0; k < COUT / 32; ++k) sred[warp][32 * k + lane] = make_float2(st_s[k], st_q[k]);
+    for (int k = 0; k < kChunks; ++k)
+      if (32 * k + lane < COUT) sred[warp][32 * k + lane] = make_float2(st_s[k], st_q[k]);
     __syncthreads();
     for (int c = threadIdx.x; c < COUT; c += blockDim.x) {
       const float2 a = sred[0][c], b = sred[1][c], cc = sred[2][c], d = sred[3][c];
@@ -292,10 +295,11 @@ static int conv_first_fwd_impl(const float* x, const float* w, void* y, int ldy,
   if (blocks > cap) blocks = cap;
   __nv_bfloat16* yy = reinterpret_cast<__nv_bfloat16*>(y);
   switch (Cout) {
+    case 16: B2_LAUNCH(conv_first_fwd_kernel<16>, (unsigned)blocks, 128, 0, stream, x, w, yy, N, D, H, W, ldy, y_coff, relu, stat_acc); break;
     case 32: B2_LAUNCH(conv_first_fwd_kernel<32>, (unsigned)blocks, 128, 0, stream, x, w, yy, N, D, H, W, ldy, y_coff, relu, stat_acc); break;
     case 64: B2_LAUNCH(conv_first_fwd_kernel<64>, (unsigned)blocks, 128, 0, stream, x, w, yy, N, D, H, W, ldy, y_coff, relu, stat_acc); break;
     default:
-      set_error("b2_conv3d_first_fwd: Cout=%d unsupported (32 or 64)", Cout);
+      set_error("b2_conv3d_first_fwd: Cout=%d unsupported (16, 32 or 64)", Cout);
       return B2_ERR_UNSUPPORTED;
   }
   B2_CHECK_CUDA(cudaGetLastError());
@@ -324,7 +328,7 @@ extern "C" int b2_conv3d_first_wgrad(const float* x, const void* dy, int lddy, i
                                      long long workspace_bytes, int N, int D, int H, int W, int Cout,
                                      cudaStream_t stream) {
   B2_REQUIRE(x && dy && dw && workspace, "b2_conv3d_first_wgrad: null pointer");
-  B2_REQUIRE(Cout == 32 || Cout == 64, "b2_conv3d_first_wgrad: Cout=%d unsupported (32 or 64)", Cout);
+  B2_REQUIRE(Cout == 16 || Cout == 32 || Cout == 64, "b2_conv3d_first_wgrad: Cout=%d unsupported (16, 32 or 64)", Cout);
   B2_REQUIRE(workspace_bytes >= b2_conv3d_first_wgrad_workspace_bytes(Cout), "b2_conv3d_first_wgrad: workspace too small");
   B2_REQUIRE(D < 1024 && H < 1024 && W < 1024 && (long long)N * D * H * W < (1LL << 31),
              "b2_conv3d_first_wgrad: volume %dx%dx%dx%d too large", N, D, H, W);
@@ -335,7 +339,9 @@ extern "C" int b2_conv3d_first_wgrad(const float* x, const void* dy, int lddy, i
   const int blocks = (int)((V + per_block - 1) / per_block);
   B2_REQUIRE(lddy % 8 == 0 && dy_coff % 8 == 0, "b2_conv3d_first_wgrad: lddy/dy_coff must be multiples of 8");
   auto* dyb = reinterpret_cast<const __nv_bfloat16*>(dy);
-  if (Cout == 32)
+  if (Cout == 16)
+    B2_LAUNCH(conv_first_wgrad_kernel<16>, blocks, 256, 0, stream, x, dyb, lddy, dy_coff, partial, N, D, H, W, per_block);
+  else if (Cout == 32)
     B2_LAUNCH(conv_first_wgrad_kernel<32>, blocks, 256, 0, stream, x, dyb, lddy, dy_coff, partial, N, D, H, W, per_block);
   else
     B2_LAUNCH(conv_first_wgrad_kernel<64>, blocks, 256, 0, stream, x, dyb, lddy, dy_coff, partial, N, D, H, W, per_block);

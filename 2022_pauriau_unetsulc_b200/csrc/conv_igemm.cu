@@ -16,6 +16,10 @@
 // the even warp of the pair loads the A box, the odd warp the weight tile.
 // Round 2: the HALO instantiation (64-channel chunks, one-plane tile boxes) loads each A tile once per (d, w) tap pair
 // with an h-halo and takes the three h taps from it by descriptor offsets; see the comment above the kernel.
+// 32-filter networks: KC = 16 (32-byte rows, 32B swizzle) for Cin = 16 and the 48-channel split operands of the exact
+// path, and N tiles of 16 x odd channels for 16-channel outputs (encoders.0.conv2 dgrad, the exact path's first
+// layer) and 48-channel ones (the dgrad shape of a 48-channel input).  16-channel
+// activations are not padded to 32: that would double the operand bytes and MMAs of those layers.
 #include "common.h"
 #include "ptx.cuh"
 #include <stdlib.h>
@@ -199,7 +203,7 @@ conv3d_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
   } else if (warp == 0) {
     // ------------------------------------------------------------------ MMA issuer
     const uint32_t idesc = make_idesc_bf16(128, (uint32_t)p.BN, 0, 0);
-    constexpr uint32_t kLayout = (KC == 64) ? SWZ_128B : SWZ_64B;
+    constexpr uint32_t kLayout = (KC == 64) ? SWZ_128B : (KC == 32 ? SWZ_64B : SWZ_32B);
     constexpr uint32_t kSbo = 8u * KC * 2u;
     const uint64_t desc_hi = make_smem_desc(0, 16, kSbo, kLayout);           // everything but the start address
     const uint32_t a0 = smem_u32(smem_a) >> 4, b0 = smem_u32(smem_b) >> 4;   // encoded start addresses of stage 0
@@ -298,6 +302,9 @@ conv3d_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       for (int chunk = 0; chunk < 8; ++chunk) {
         const int c0 = chunk * 32;
         if (c0 >= p.BN) break;
+        // 16 in the last chunk when BN = 16 x odd: columns 16..31 are not this tile's.  Only the stores are cut to them;
+        // the statistics of those columns land in lanes 16..31 of the column sums, which are never committed.
+        const int ncol = p.BN - c0 < 32 ? p.BN - c0 : 32;
         uint32_t v[32];
         tmem_ld32(t_addr + c0, v);
         tmem_ld_wait();
@@ -316,7 +323,7 @@ conv3d_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
               uint4 u = make_uint4(0, 0, 0, 0);
-              if (valid) u = __ldg(rp + j);
+              if (valid) u = __ldg(rp + (j & ((ncol >> 3) - 1)));   // ncol = 16: columns 16..31 re-read 0..15
               const uint32_t wds[4] = {u.x, u.y, u.z, u.w};
 #pragma unroll
               for (int e = 0; e < 4; ++e) {
@@ -335,6 +342,7 @@ conv3d_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
             float4* dst = reinterpret_cast<float4*>(y32 + vox * p.ldy + p.y_coff + n0 + c0);
 #pragma unroll
             for (int j = 0; j < 8; ++j) {
+              if (4 * j >= ncol) break;
               float4 o;
               o.x = __uint_as_float(v[4 * j + 0]);
               o.y = __uint_as_float(v[4 * j + 1]);
@@ -349,6 +357,7 @@ conv3d_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
             uint4* dst = reinterpret_cast<uint4*>(p.y + vox * p.ldy + p.y_coff + n0 + c0);
 #pragma unroll
             for (int j = 0; j < 4; ++j) {
+              if (8 * j >= ncol) break;
               float f[8];
 #pragma unroll
               for (int e = 0; e < 8; ++e) {
@@ -373,7 +382,7 @@ conv3d_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
       float2* sbuf = reinterpret_cast<float2*>(smem_a);   // [4][Cout]
 #pragma unroll
       for (int chunk = 0; chunk < 8; ++chunk)
-        if (chunk * 32 < p.BN) sbuf[q * p.Cout + chunk * 32 + lane] = make_float2(st_s[chunk], st_q[chunk]);
+        if (chunk * 32 + lane < p.BN) sbuf[q * p.Cout + chunk * 32 + lane] = make_float2(st_s[chunk], st_q[chunk]);
       asm volatile("bar.sync 1, 128;" ::: "memory");
       for (int c = q * 32 + lane; c < p.Cout; c += 128) {
         const float2 a = sbuf[c], b = sbuf[p.Cout + c], cc = sbuf[2 * p.Cout + c], d = sbuf[3 * p.Cout + c];
@@ -702,8 +711,8 @@ static int conv3d_igemm_impl(const void* x, int ldx, int x_coff, const void* wpa
                              long long splitk_workspace_bytes, cudaStream_t stream) {
   B2_REQUIRE(x && wpack && y, "b2_conv3d_igemm: null pointer");
   B2_REQUIRE(N > 0 && D > 0 && H > 0 && W > 0, "b2_conv3d_igemm: bad shape %dx%dx%dx%d", N, D, H, W);
-  B2_REQUIRE(Cin % 32 == 0 && Cin >= 32, "b2_conv3d_igemm: Cin=%d must be a multiple of 32", Cin);
-  B2_REQUIRE(Cout % 32 == 0 && Cout >= 32, "b2_conv3d_igemm: Cout=%d must be a multiple of 32", Cout);
+  B2_REQUIRE(Cin % 16 == 0 && Cin >= 16, "b2_conv3d_igemm: Cin=%d must be a multiple of 16", Cin);
+  B2_REQUIRE(Cout % 16 == 0 && Cout >= 16, "b2_conv3d_igemm: Cout=%d must be a multiple of 16", Cout);
   B2_REQUIRE(ldx % 8 == 0 && x_coff % 8 == 0 && ldy % 8 == 0 && y_coff % 8 == 0,
              "b2_conv3d_igemm: channel strides/offsets must be multiples of 8");
   B2_REQUIRE(x_coff + Cin <= ldx && y_coff + Cout <= ldy, "b2_conv3d_igemm: channel window out of range");
@@ -719,14 +728,17 @@ static int conv3d_igemm_impl(const void* x, int ldx, int x_coff, const void* wpa
   p.tiles_w = ceil_div(W, p.bw);
   p.tiles_h = ceil_div(H, p.bh);
   p.tiles_d = ceil_div(D, p.bd);
-  // N tile: largest divisor of Cout that is a multiple of 32 and <= 256
+  // N tile: largest divisor of Cout that is a multiple of 32 and <= 256; for Cout = 16 x odd (16, 48, ...) the largest
+  // such divisor that is a multiple of 16 (the epilogue stores the last 16 columns of a 32-column chunk alone)
   int BN = 0;
   for (int c = 256; c >= 32; c -= 32)
     if (Cout % c == 0) { BN = c; break; }
+  for (int c = 256; BN == 0 && c >= 16; c -= 16)
+    if (Cout % c == 0) BN = c;
   B2_REQUIRE(BN > 0, "b2_conv3d_igemm: no N tile for Cout=%d", Cout);
   p.BN = BN;
   p.n_tiles_n = Cout / BN;
-  p.KC = (Cin % 64 == 0) ? 64 : 32;
+  p.KC = (Cin % 64 == 0) ? 64 : (Cin % 32 == 0 ? 32 : 16);
   p.n_chunks = Cin / p.KC;
   p.a_bytes = 128 * p.KC * 2;
   p.b_bytes = BN * p.KC * 2;
@@ -848,10 +860,14 @@ static int conv3d_igemm_impl(const void* x, int ldx, int x_coff, const void* wpa
     B2_CHECK_CUDA(cudaFuncSetAttribute((conv3d_igemm_kernel<64, false>), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        227 * 1024));
     B2_LAUNCH((conv3d_igemm_kernel<64, false>), (unsigned)grid, kThreads, smem_bytes, stream, ta, tb, p);
-  } else {
+  } else if (p.KC == 32) {
     B2_CHECK_CUDA(cudaFuncSetAttribute((conv3d_igemm_kernel<32, false>), cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        227 * 1024));
     B2_LAUNCH((conv3d_igemm_kernel<32, false>), (unsigned)grid, kThreads, smem_bytes, stream, ta, tb, p);
+  } else {
+    B2_CHECK_CUDA(cudaFuncSetAttribute((conv3d_igemm_kernel<16, false>), cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       227 * 1024));
+    B2_LAUNCH((conv3d_igemm_kernel<16, false>), (unsigned)grid, kThreads, smem_bytes, stream, ta, tb, p);
   }
   B2_CHECK_CUDA(cudaGetLastError());
   if (p.splits > 1) {

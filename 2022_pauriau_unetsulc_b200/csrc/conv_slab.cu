@@ -146,7 +146,7 @@ conv3d_slab_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
         }
   } else if (warp == 0) {
     // ---------------------------------------------------------------- MMA issuer
-    constexpr uint32_t kLayout = (KC == 64) ? SWZ_128B : SWZ_64B;
+    constexpr uint32_t kLayout = (KC == 64) ? SWZ_128B : (KC == 32 ? SWZ_64B : SWZ_32B);
     constexpr uint32_t kSbo = 8u * kRowBytes;
     const uint64_t desc_hi = make_smem_desc(0, 16, kSbo, kLayout);
     const uint32_t p0 = smem_u32(smem_p) >> 4, b0 = smem_u32(smem_b) >> 4;
@@ -329,10 +329,12 @@ static long long slab_padded(int D, int H, int W, int tw) {
 }
 static int slab_tile_w(int D, int H, int W) { return slab_padded(D, H, W, 16) < slab_padded(D, H, W, 32) ? 16 : 32; }
 
+// Cin: 16 (encoders.0.conv2 of a 32-filter network, one 16-channel chunk) or a multiple of 32 (decoders.2.conv1 of a
+// 32-filter network has Cin = 96: three 32-channel chunks).
 bool slab_applicable(int N, int D, int H, int W, int Cin, int Cout, int y_is_fp32) {
   if (y_is_fp32) return false;
   if (!(Cout == 32 || Cout == 64)) return false;
-  if (!(Cin % 64 == 0 || Cin == 32)) return false;
+  if (!(Cin % 32 == 0 || Cin == 16)) return false;
   const long long padded = slab_padded(D, H, W, slab_tile_w(D, H, W));
   if (padded * 100 > (long long)W * H * D * 150) return false;
   return true;
@@ -353,7 +355,7 @@ int launch_slab(const void* x, int ldx, int x_coff, const void* wpack, void* y, 
                 cudaStream_t stream) {
   SlabParams p;
   p.N = N; p.D = D; p.H = H; p.W = W; p.Cin = Cin; p.Cout = Cout;
-  const int KC = (Cin % 64 == 0) ? 64 : 32;
+  const int KC = (Cin % 64 == 0) ? 64 : (Cin % 32 == 0 ? 32 : 16);
   const int tw = slab_tile_w(D, H, W), th = 128 / tw;
   p.n_chunks = Cin / KC;
   p.tiles_w = ceil_div(W, tw);
@@ -386,8 +388,10 @@ int launch_slab(const void* x, int ldx, int x_coff, const void* wpack, void* y, 
   const size_t smem_bytes = 2 * (size_t)b_bytes + (size_t)p.stages * plane_bytes + 1024 + 512;
   if (KC == 64) return tw == 32 ? launch_slab_t<64, 32>(ta, tb, p, smem_bytes, stream)
                                 : launch_slab_t<64, 16>(ta, tb, p, smem_bytes, stream);
-  return tw == 32 ? launch_slab_t<32, 32>(ta, tb, p, smem_bytes, stream)
-                  : launch_slab_t<32, 16>(ta, tb, p, smem_bytes, stream);
+  if (KC == 32) return tw == 32 ? launch_slab_t<32, 32>(ta, tb, p, smem_bytes, stream)
+                                : launch_slab_t<32, 16>(ta, tb, p, smem_bytes, stream);
+  return tw == 32 ? launch_slab_t<16, 32>(ta, tb, p, smem_bytes, stream)
+                  : launch_slab_t<16, 16>(ta, tb, p, smem_bytes, stream);
 }
 
 }  // namespace b2

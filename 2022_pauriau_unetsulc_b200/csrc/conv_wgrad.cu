@@ -14,6 +14,8 @@
 // Round 2 added two planning modes (plan_wgrad): the "dY-halo" mode for Cout <= 128 at one-plane tile boxes — X is
 // shifted only in (d, w), the three h taps are three N atoms of ONE dY tile loaded with an h-halo (N = 192 per MMA) —
 // and stream-K runs when a uniform K split would leave SMs idle (wgrad_segment).
+// 32-filter networks add Cin = 16 slots (32-byte rows, 32B swizzle, 8 slots per 128-row group) and Cout = 32 dY tiles
+// (64-byte rows, 64B swizzle; in halo mode three 32-channel atoms, N = 96).
 #include "common.h"
 #include "ptx.cuh"
 #include <stdlib.h>
@@ -35,7 +37,7 @@ struct WgradParams {
   long long ksteps_total;
   int stages_a, n_prod;   // ring depth (a multiple of n_prod) and number of active slot-group producers
   int a_bytes, b_bytes, slot_bytes;
-  int halo;        // "dY-halo" mode (64-channel N tiles read as three h-shifted atoms): see plan_wgrad
+  int halo;        // "dY-halo" mode (BN-channel N tiles read as three h-shifted atoms): see plan_wgrad
   int d_fast;      // K-step order (w, d, h) instead of (w, h, d): see wgrad_tile
   int stages_b;    // depth of the fixed-operand ring (2-4)
   int grid;        // CTAs launched
@@ -203,12 +205,13 @@ conv3d_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_con
         mbar_wait(&empty_b[sb], pb ^ 1);
         if (elect_one()) {
           mbar_arrive_expect_tx(&full_b[sb], (uint32_t)p.b_bytes);
-          if (p.halo) {   // one box with an h-halo: (bh + 2) lines of bw voxels x 64 channels, zero-filled outside
+          if (p.halo) {   // one box with an h-halo: (bh + 2) lines of bw voxels x BN channels, zero-filled outside
             tma_load_5d(smem_b + (size_t)sb * p.b_bytes, &tmap_dy, &full_b[sb], n0, w0, h0 - 1, d0, n);
-          } else {
-            for (int j = 0; j < p.BN / 64; ++j)
-              tma_load_5d(smem_b + (size_t)sb * p.b_bytes + (size_t)j * 16384, &tmap_dy, &full_b[sb], n0 + j * 64, w0,
-                          h0, d0, n);
+          } else {   // 64-channel boxes of 128 voxels (one 32-channel box when BN = 32)
+            const int box_c = p.BN < 64 ? p.BN : 64;
+            for (int j = 0; j < p.BN / box_c; ++j)
+              tma_load_5d(smem_b + (size_t)sb * p.b_bytes + (size_t)j * 128 * box_c * 2, &tmap_dy, &full_b[sb],
+                          n0 + j * box_c, w0, h0, d0, n);
           }
         }
         __syncwarp();
@@ -216,17 +219,20 @@ conv3d_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_con
       }
     }
   } else if (warp == 0) {
-    // halo mode: N = 3 x 64 — the three N atoms are the SAME dY tile shifted by -1 / 0 / +1 h-lines (atom stride = one
+    // halo mode: N = 3 x BN — the three N atoms are the SAME dY tile shifted by -1 / 0 / +1 h-lines (atom stride = one
     // h-line of bw voxel rows), i.e. one MMA accumulates the three h taps of the slot pair: 6 taps per instruction,
-    // 10 KB of shared-memory reads for 96 tensor-cycles instead of 6 KB for 32
-    const uint32_t acc_cols = p.halo ? 192u : (uint32_t)p.BN;
+    // 10 KB of shared-memory reads for 96 tensor-cycles instead of 6 KB for 32 (BN = 64)
+    const uint32_t acc_cols = p.halo ? 3u * (uint32_t)p.BN : (uint32_t)p.BN;
     const uint32_t idesc = make_idesc_bf16(128, acc_cols, 1, 1);
-    const uint32_t layout_a = (p.SWC == 64) ? SWZ_128B : SWZ_64B;
+    const uint32_t layout_a = (p.SWC == 64) ? SWZ_128B : (p.SWC == 32 ? SWZ_64B : SWZ_32B);
     const uint32_t row_a = (uint32_t)p.SWC * 2u;
     const uint64_t a_hi = make_smem_desc(0, (uint32_t)p.slot_bytes, 8 * row_a, layout_a);
-    const uint64_t b_hi = make_smem_desc(0, p.halo ? (uint32_t)p.bw * 128u : 16384u, 1024, SWZ_128B);
+    // dY rows: 64-channel atoms (128 B, 128B swizzle) or, for BN = 32, one 32-channel atom (64 B, 64B swizzle)
+    const uint32_t row_b = p.BN < 64 ? (uint32_t)p.BN * 2u : 128u;
+    const uint64_t b_hi = make_smem_desc(0, p.halo ? (uint32_t)p.bw * row_b : 128u * row_b, 8 * row_b,
+                                         row_b == 128u ? SWZ_128B : SWZ_64B);
     const uint32_t a0 = smem_u32(smem_a) >> 4, b0 = smem_u32(smem_b) >> 4;
-    const uint32_t a_kstep = (16 * row_a) >> 4, b_kstep = (16 * 128) >> 4;   // encoded advance per K16 (16 voxels)
+    const uint32_t a_kstep = (16 * row_a) >> 4, b_kstep = (16 * row_b) >> 4;   // encoded advance per K16 (16 voxels)
     int sa = 0, sb = 0;
     uint32_t pa = 0, pb = 0;
     for (int sg = 0; wgrad_segment(p, sg, seg); ++sg) {
@@ -274,16 +280,16 @@ conv3d_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_con
         const bool valid = s < p.total_slots;
         const int tap = s / p.n_cchunks;
         const int ci = (s % p.n_cchunks) * p.SWC + row % p.SWC;
-        const uint32_t acc_cols = p.halo ? 192u : (uint32_t)p.BN;
+        const uint32_t acc_cols = p.halo ? 3u * (uint32_t)p.BN : (uint32_t)p.BN;
         const uint32_t t_addr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(g - g_begin) * acc_cols;
         for (int c0 = 0; c0 < (int)acc_cols; c0 += 32) {
           uint32_t v[32];
           tmem_ld32(t_addr + c0, v);
           tmem_ld_wait();
           if (valid) {
-            // halo mode: accumulator columns [64 j, 64 j + 64) = h tap dh = 1 - j of the slot's (dd, dw) shift
-            const int full_tap = p.halo ? (tap / 3) * 9 + (2 - c0 / 64) * 3 + tap % 3 : tap;
-            const int col = p.halo ? (c0 & 63) : c0;
+            // halo mode: accumulator columns [BN j, BN j + BN) = h tap dh = 1 - j of the slot's (dd, dw) shift
+            const int full_tap = p.halo ? (tap / 3) * 9 + (2 - c0 / p.BN) * 3 + tap % 3 : tap;
+            const int col = p.halo ? (c0 % p.BN) : c0;
             float4* d4 = reinterpret_cast<float4*>(p.ws + (((size_t)seg.layer * 27 + full_tap) * p.Cin + ci) * p.Cout +
                                                    n0 + col);
 #pragma unroll
@@ -540,9 +546,9 @@ static int plan_wgrad(WgradParams& p, int N, int D, int H, int W, int Cin, int C
   p.tiles_w = ceil_div(W, p.bw);
   p.tiles_h = ceil_div(H, p.bh);
   p.tiles_d = ceil_div(D, p.bd);
-  p.SWC = (Cin % 64 == 0) ? 64 : 32;
+  p.SWC = (Cin % 64 == 0) ? 64 : (Cin % 32 == 0 ? 32 : 16);
   p.n_cchunks = Cin / p.SWC;
-  p.BN = (Cout % 256 == 0) ? 256 : (Cout % 192 == 0 ? 192 : (Cout % 128 == 0 ? 128 : 64));
+  p.BN = (Cout % 256 == 0) ? 256 : (Cout % 192 == 0 ? 192 : (Cout % 128 == 0 ? 128 : (Cout % 64 == 0 ? 64 : 32)));
   p.n_cout_tiles = Cout / p.BN;
   // "dY-halo" mode for Cout <= 128 at one-plane tile boxes (decoders.2.conv2, encoders.0.conv2, encoders.1.*,
   // decoders.1.*: round 1 ran the Cout = 64 ones at 640-790 TFLOP/s, bound by re-loading the shifted operand 27 times
@@ -554,17 +560,18 @@ static int plan_wgrad(WgradParams& p, int N, int D, int H, int W, int Cin, int C
   // 86 -> 67.
   static const bool no_halo = getenv("B2_NO_WGRAD_HALO") != nullptr;
   static const int halo_max_c = getenv("B2_WGRAD_HALO_MAXC") ? atoi(getenv("B2_WGRAD_HALO_MAXC")) : 128;
-  p.halo = (allow_halo && !no_halo && Cout % 64 == 0 && Cout <= halo_max_c && p.bd == 1 && p.bw % 8 == 0) ? 1 : 0;
-  if (p.halo) {   // 64-channel N tiles, each read as three h-shifted atoms
-    p.BN = 64;
-    p.n_cout_tiles = Cout / 64;
+  p.halo = (allow_halo && !no_halo && Cout % 32 == 0 && Cout <= halo_max_c && p.bd == 1 && p.bw % 8 == 0) ? 1 : 0;
+  if (p.halo) {   // 64-channel N tiles (32 when Cout = 32), each read as three h-shifted atoms
+    p.BN = (Cout % 64 == 0) ? 64 : 32;
+    p.n_cout_tiles = Cout / p.BN;
   }
   static const bool plane_order = getenv("B2_WGRAD_PLANE_ORDER") != nullptr;
   p.d_fast = (p.halo && !plane_order) ? 1 : 0;
   p.total_slots = (p.halo ? 9 : 27) * p.n_cchunks;
   p.SPG = 128 / p.SWC;
   p.G = ceil_div(p.total_slots, p.SPG);
-  const int P = p.halo ? 2 : 512 / p.BN;   // accumulators per CTA (one group per CTA measured slower: 237 vs 211 us)
+  // accumulators per CTA (one group per CTA measured slower: 237 vs 211 us); halo: 2 at BN = 64, 5 at BN = 32
+  const int P = 512 / (p.halo ? 3 * p.BN : p.BN);
   p.n_gchunks = ceil_div(p.G, P);
   p.gpc = ceil_div(p.G, p.n_gchunks);
   p.n_gchunks = ceil_div(p.G, p.gpc);
@@ -591,7 +598,7 @@ static int plan_wgrad(WgradParams& p, int N, int D, int H, int W, int Cin, int C
   }
   p.slot_bytes = 128 * p.SWC * 2;
   p.a_bytes = 128 * 128 * 2;
-  p.b_bytes = p.halo ? (p.bh + 2) * p.bw * 128 : 128 * p.BN * 2;
+  p.b_bytes = p.halo ? (p.bh + 2) * p.bw * p.BN * 2 : 128 * p.BN * 2;
   const int budget = 227 * 1024 - 1024 - 512;
   p.stages_a = (budget - 2 * p.b_bytes) / p.a_bytes;
   if (p.stages_a > 4) p.stages_a = 4;
@@ -610,8 +617,13 @@ static int plan_wgrad(WgradParams& p, int N, int D, int H, int W, int Cin, int C
 
 using namespace b2;
 
+// Cin = 16 or a multiple of 32 (shifted slots of 16, 32 or 64 channels), Cout a multiple of 32
+static bool wgrad_shape_ok(int Cin, int Cout) {
+  return (Cin == 16 || (Cin % 32 == 0 && Cin >= 32)) && Cout % 32 == 0 && Cout >= 32;
+}
+
 extern "C" long long b2_conv3d_wgrad_workspace_bytes(int N, int D, int H, int W, int Cin, int Cout) {
-  if (Cin % 32 != 0 || Cout % 64 != 0 || N <= 0 || D <= 0 || H <= 0 || W <= 0) return -1;
+  if (!wgrad_shape_ok(Cin, Cout) || N <= 0 || D <= 0 || H <= 0 || W <= 0) return -1;
   WgradParams p;
   const bool swap = wgrad_swap_roles(Cin, Cout);
   if (plan_wgrad(p, N, D, H, W, swap ? Cout : Cin, swap ? Cin : Cout, !swap) != 0) return -1;
@@ -623,8 +635,8 @@ static int wgrad_partial_impl(const void* x, int ldx, int x_coff, const void* dy
                               WgradParams& p, bool& swap, cudaStream_t stream) {
   B2_REQUIRE(x && dy && workspace, "b2_conv3d_wgrad: null pointer");
   B2_REQUIRE(N > 0 && D > 0 && H > 0 && W > 0, "b2_conv3d_wgrad: bad shape");
-  B2_REQUIRE(Cin % 32 == 0 && Cin >= 32, "b2_conv3d_wgrad: Cin=%d must be a multiple of 32", Cin);
-  B2_REQUIRE(Cout % 64 == 0 && Cout >= 64, "b2_conv3d_wgrad: Cout=%d must be a multiple of 64", Cout);
+  B2_REQUIRE(wgrad_shape_ok(Cin, Cout), "b2_conv3d_wgrad: Cin=%d must be 16 or a multiple of 32, Cout=%d a multiple of 32",
+             Cin, Cout);
   B2_REQUIRE(ldx % 8 == 0 && x_coff % 8 == 0 && ldy % 8 == 0 && y_coff % 8 == 0,
              "b2_conv3d_wgrad: channel strides/offsets must be multiples of 8");
   swap = wgrad_swap_roles(Cin, Cout);
@@ -642,7 +654,8 @@ static int wgrad_partial_impl(const void* x, int ldx, int x_coff, const void* dy
   CUtensorMap tx, ty;
   int rc = make_act_tmap(&tx, sh_ptr, N, D, H, W, sh_c, sh_ld, sh_off, p.SWC, p.bw, p.bh, p.bd);
   if (rc) return rc;
-  rc = make_act_tmap(&ty, fx_ptr, N, D, H, W, fx_c, fx_ld, fx_off, 64, p.bw, p.halo ? p.bh + 2 : p.bh, p.bd);
+  rc = make_act_tmap(&ty, fx_ptr, N, D, H, W, fx_c, fx_ld, fx_off, p.BN < 64 ? p.BN : 64, p.bw,
+                     p.halo ? p.bh + 2 : p.bh, p.bd);
   if (rc) return rc;
 
   const size_t smem_bytes = (size_t)p.stages_b * p.b_bytes + (size_t)p.stages_a * p.a_bytes + 1024 + 512;

@@ -126,9 +126,12 @@ __global__ void __launch_bounds__(256) pack_weights_multi_kernel(const PackArgs 
   if (Cin % 64 == 0) {
     const int ci_tiles = Cin / 64;
     pack_tile<64>(a.w[l], a.wf[l], a.wd[l], Cout, Cin, (b / ci_tiles) * kPkCo, (b % ci_tiles) * 64, tile);
-  } else {
+  } else if (Cin % 32 == 0) {
     const int ci_tiles = Cin / 32;
     pack_tile<32>(a.w[l], a.wf[l], a.wd[l], Cout, Cin, (b / ci_tiles) * kPkCo, (b % ci_tiles) * 32, tile);
+  } else {   // Cin = 16 (encoders.0.conv2 of a 32-filter network) or 48 (its split operand in exact mode)
+    const int ci_tiles = Cin / 16;
+    pack_tile<16>(a.w[l], a.wf[l], a.wd[l], Cout, Cin, (b / ci_tiles) * kPkCo, (b % ci_tiles) * 16, tile);
   }
 }
 
@@ -187,10 +190,9 @@ extern "C" int b2_pack_conv_weights_multi(const float* const* w, void* const* wf
       a.cout[k] = cout[i];
       a.cin[k] = cin[i];
       a.first_block[k] = blocks;
-      B2_REQUIRE(cout[i] % kPkCo == 0 && cin[i] % 32 == 0,
-                 "b2_pack_conv_weights_multi: layer %d: Cout=%d must be a multiple of 16 and Cin=%d of 32", i, cout[i],
-                 cin[i]);
-      blocks += (cout[i] / kPkCo) * (cin[i] % 64 == 0 ? cin[i] / 64 : cin[i] / 32);
+      B2_REQUIRE(cout[i] % kPkCo == 0 && cin[i] % 16 == 0 && cin[i] > 0,
+                 "b2_pack_conv_weights_multi: layer %d: Cout=%d and Cin=%d must be multiples of 16", i, cout[i], cin[i]);
+      blocks += (cout[i] / kPkCo) * (cin[i] % 64 == 0 ? cin[i] / 64 : (cin[i] % 32 == 0 ? cin[i] / 32 : cin[i] / 16));
       ++k;
     }
     a.first_block[k] = blocks;

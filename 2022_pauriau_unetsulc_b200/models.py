@@ -99,9 +99,10 @@ class UNet3D(nn.Module):
         if dropout not in (0, 0., None):
             raise ValueError("unetsulc_b200.UNet3D: dropout=%r unsupported (reference passes 0.)" % dropout)
         f = init_channel_number
-        if f != 64:
-            raise ValueError("unetsulc_b200.UNet3D: init_channel_number=%r unsupported (64 only: the tcgen05 conv "
-                             "kernels need channel counts that are multiples of 32/64)" % f)
+        if f not in (32, 64):
+            raise ValueError("unetsulc_b200.UNet3D: init_channel_number=%r unsupported (32 or 64: the tcgen05 conv "
+                             "kernels take 16-channel operands at the narrowest, and the statistics accumulators at "
+                             "most 512 channels)" % (f,))
         g = min(f // 2, 32)
         self.num_groups = g
         self.init_channel_number = f

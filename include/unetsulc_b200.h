@@ -28,7 +28,8 @@ const char* b2_last_error(void);
 
 /* ---- 3x3x3 stride-1 pad-1 Conv3d (the 14 convs inside deepsulci UNet3D; training.py:206, 211) -------------------
  * Implicit GEMM on tcgen05/TMEM fed by TMA.  fprop: x = layer input, wpack = fprop pack, relu=1.
- * dgrad: x = dY, wpack = dgrad pack, Cin/Cout swapped, relu=0.  y_is_fp32 selects a fp32 output buffer.      */
+ * dgrad: x = dY, wpack = dgrad pack, Cin/Cout swapped, relu=0.  y_is_fp32 selects a fp32 output buffer.
+ * Cin and Cout: multiples of 16 (K chunks of 64, 32 or 16 channels; N tiles of up to 256 channels).               */
 int b2_conv3d_igemm(const void* x, int ldx, int x_coff, const void* wpack, void* y, int ldy, int y_coff,
                     int y_is_fp32, int N, int D, int H, int W, int Cin, int Cout, int relu, cudaStream_t stream);
 
@@ -63,7 +64,8 @@ int b2_relu_gn_bwd_acc(const long long* stat_acc, const void* dy, int lddy, int 
                        float* dbeta, void* workspace, long long workspace_bytes, const long long* dy_row_labels,
                        cudaStream_t stream);   /* dy_row_labels (may be NULL): see b2_head_ce_bstats */
 
-/* dW[co][ci][3][3][3] (fp32, PyTorch layout) = sum_v dY[v,co] * X[v+off,ci]                                      */
+/* dW[co][ci][3][3][3] (fp32, PyTorch layout) = sum_v dY[v,co] * X[v+off,ci].  Cin: 16 or a multiple of 32; Cout: a
+ * multiple of 32.  The workspace query returns -1 for any other shape.                                             */
 long long b2_conv3d_wgrad_workspace_bytes(int N, int D, int H, int W, int Cin, int Cout);
 int b2_conv3d_wgrad(const void* x, int ldx, int x_coff, const void* dy, int ldy, int y_coff, float* dw,
                     void* workspace, long long workspace_bytes, int N, int D, int H, int W, int Cin, int Cout,
@@ -79,7 +81,8 @@ int b2_conv3d_wgrad_partial(const void* x, int ldx, int x_coff, const void* dy, 
 int b2_wgrad_reduce_multi(const float* const* ws, float* const* dw, const int* splits, const int* cin,
                           const int* cout, const int* swapped, int count, cudaStream_t stream);
 
-/* encoders.0.conv1 (Cin = 1): direct convolution on the fp32 [N,D,H,W] skeleton volume (dataset.py:78-80)        */
+/* encoders.0.conv1 (Cin = 1): direct convolution on the fp32 [N,D,H,W] skeleton volume (dataset.py:78-80).
+ * Cout = 16, 32 or 64 (init_channel_number 32 or 64).                                                              */
 int b2_conv3d_first_fwd(const float* x, const float* w, void* y, int ldy, int y_coff, int N, int D, int H, int W,
                         int Cout, int relu, cudaStream_t stream);
 /* same, with the GroupNorm statistics of the stored output fused in (batch 1): stat_acc int64 [Cout][4], see above  */
