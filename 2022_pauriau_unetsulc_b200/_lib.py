@@ -20,6 +20,13 @@ SIGNATURES = {
     "b2_conv3d_igemm_bstats": (_i, [_vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
     "b2_relu_gn_finalize_acc": (_i, [_vp, _ll, _i, _i, _f, _vp, _vp, _vp, _vp, _vp]),
     "b2_relu_gn_bwd_acc": (_i, [_vp, _vp, _i, _i, _vp, _ll, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _vp, _vp]),
+    "b2_conv3d_igemm_bias": (_i, [_vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _ll,
+                                  _vp]),
+    "b2_conv3d_first_fwd_bias": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp]),
+    "b2_relu_gn_bwd_dbias": (_i, [_vp, _i, _i, _vp, _i, _ll, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _vp, _vp, _vp,
+                                  _vp]),
+    "b2_relu_gn_bwd_acc_dbias": (_i, [_vp, _vp, _i, _i, _vp, _ll, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _ll, _vp, _vp,
+                                      _vp, _vp]),
     "b2_conv3d_wgrad_workspace_bytes": (_ll, [_i, _i, _i, _i, _i, _i]),
     "b2_conv3d_wgrad": (_i, [_vp, _i, _i, _vp, _i, _i, _vp, _vp, _ll, _i, _i, _i, _i, _i, _i, _vp]),
     "b2_conv3d_wgrad_partial": (_i, [_vp, _i, _i, _vp, _i, _i, _vp, _ll, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),

@@ -14,15 +14,20 @@ namespace b2 {
 // channel, sum and sum of squares of the STORED (ReLU'd, bf16-rounded) outputs — the GroupNorm statistics — into
 // the exact [COUT][4] accumulators of common.h (one atomic add per block and channel).  COUT = 16 (32-filter networks)
 // sums one half-empty 32-column chunk: lanes 16..31 carry zeros and are not stored.
+// bias (fp32 [COUT], may be NULL) is added to the accumulator before ReLU: a voxel whose 27 neighbours are all zero
+// (every tap skipped) stores relu(bias) and contributes it to the statistics.
 template <int COUT>
 __global__ void __launch_bounds__(128)
 conv_first_fwd_kernel(const float* __restrict__ x, const float* __restrict__ w /*[COUT][27]*/,
                       __nv_bfloat16* __restrict__ y, int N, int D, int H, int W, int ldy, int y_coff, int relu,
-                      long long* __restrict__ stat_acc) {
+                      long long* __restrict__ stat_acc, const float* __restrict__ bias) {
   pdl_prologue();
   __shared__ __align__(16) float ws[27][COUT];
   __shared__ float2 sred[4][COUT];
+  __shared__ float bs[COUT];
   for (int i = threadIdx.x; i < 27 * COUT; i += blockDim.x) ws[i % 27][i / 27] = w[i];  // w[co*27+tap]
+  if (bias != nullptr)
+    for (int i = threadIdx.x; i < COUT; i += blockDim.x) bs[i] = bias[i];
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const long long V = (long long)N * D * H * W;
@@ -64,6 +69,10 @@ conv_first_fwd_kernel(const float* __restrict__ x, const float* __restrict__ w /
           acc[4 * c4 + 3] = fmaf(xv[tap], q.w, acc[4 * c4 + 3]);
         }
       }
+    }
+    if (bias != nullptr) {
+#pragma unroll
+      for (int c = 0; c < COUT; ++c) acc[c] += bs[c];
     }
     if (relu) {
 #pragma unroll
@@ -286,7 +295,8 @@ static constexpr int kFirstFwdStatBlocks = 148 * 4;
 using namespace b2;
 
 static int conv_first_fwd_impl(const float* x, const float* w, void* y, int ldy, int y_coff, int N, int D, int H,
-                               int W, int Cout, int relu, long long* stat_acc, cudaStream_t stream) {
+                               int W, int Cout, int relu, long long* stat_acc, const float* bias,
+                               cudaStream_t stream) {
   B2_REQUIRE(x && w && y, "b2_conv3d_first_fwd: null pointer");
   B2_REQUIRE(ldy % 8 == 0 && y_coff % 8 == 0, "b2_conv3d_first_fwd: ldy/y_coff must be multiples of 8");
   const long long V = (long long)N * D * H * W;
@@ -295,9 +305,9 @@ static int conv_first_fwd_impl(const float* x, const float* w, void* y, int ldy,
   if (blocks > cap) blocks = cap;
   __nv_bfloat16* yy = reinterpret_cast<__nv_bfloat16*>(y);
   switch (Cout) {
-    case 16: B2_LAUNCH(conv_first_fwd_kernel<16>, (unsigned)blocks, 128, 0, stream, x, w, yy, N, D, H, W, ldy, y_coff, relu, stat_acc); break;
-    case 32: B2_LAUNCH(conv_first_fwd_kernel<32>, (unsigned)blocks, 128, 0, stream, x, w, yy, N, D, H, W, ldy, y_coff, relu, stat_acc); break;
-    case 64: B2_LAUNCH(conv_first_fwd_kernel<64>, (unsigned)blocks, 128, 0, stream, x, w, yy, N, D, H, W, ldy, y_coff, relu, stat_acc); break;
+    case 16: B2_LAUNCH(conv_first_fwd_kernel<16>, (unsigned)blocks, 128, 0, stream, x, w, yy, N, D, H, W, ldy, y_coff, relu, stat_acc, bias); break;
+    case 32: B2_LAUNCH(conv_first_fwd_kernel<32>, (unsigned)blocks, 128, 0, stream, x, w, yy, N, D, H, W, ldy, y_coff, relu, stat_acc, bias); break;
+    case 64: B2_LAUNCH(conv_first_fwd_kernel<64>, (unsigned)blocks, 128, 0, stream, x, w, yy, N, D, H, W, ldy, y_coff, relu, stat_acc, bias); break;
     default:
       set_error("b2_conv3d_first_fwd: Cout=%d unsupported (16, 32 or 64)", Cout);
       return B2_ERR_UNSUPPORTED;
@@ -308,7 +318,7 @@ static int conv_first_fwd_impl(const float* x, const float* w, void* y, int ldy,
 
 extern "C" int b2_conv3d_first_fwd(const float* x, const float* w, void* y, int ldy, int y_coff, int N, int D, int H,
                                    int W, int Cout, int relu, cudaStream_t stream) {
-  return conv_first_fwd_impl(x, w, y, ldy, y_coff, N, D, H, W, Cout, relu, nullptr, stream);
+  return conv_first_fwd_impl(x, w, y, ldy, y_coff, N, D, H, W, Cout, relu, nullptr, nullptr, stream);
 }
 
 // Same, with the GroupNorm statistics of the stored output fused in (batch 1): stat_acc int64 [Cout][4] exact
@@ -317,7 +327,16 @@ extern "C" int b2_conv3d_first_fwd_stats(const float* x, const float* w, void* y
                                          int H, int W, int Cout, int relu, long long* stat_acc, cudaStream_t stream) {
   B2_REQUIRE(stat_acc, "b2_conv3d_first_fwd_stats: null pointer");
   B2_REQUIRE(N == 1, "b2_conv3d_first_fwd_stats: fused statistics need batch 1");
-  return conv_first_fwd_impl(x, w, y, ldy, y_coff, N, D, H, W, Cout, relu, stat_acc, stream);
+  return conv_first_fwd_impl(x, w, y, ldy, y_coff, N, D, H, W, Cout, relu, stat_acc, nullptr, stream);
+}
+
+// Same with a conv bias (fp32 [Cout]) added before ReLU; stat_acc may be NULL (no statistics) and needs batch 1.
+extern "C" int b2_conv3d_first_fwd_bias(const float* x, const float* w, const float* bias, void* y, int ldy, int y_coff,
+                                        int N, int D, int H, int W, int Cout, int relu, long long* stat_acc,
+                                        cudaStream_t stream) {
+  B2_REQUIRE(bias, "b2_conv3d_first_fwd_bias: null bias");
+  B2_REQUIRE(!stat_acc || N == 1, "b2_conv3d_first_fwd_bias: fused statistics need batch 1");
+  return conv_first_fwd_impl(x, w, y, ldy, y_coff, N, D, H, W, Cout, relu, stat_acc, bias, stream);
 }
 
 extern "C" long long b2_conv3d_first_wgrad_workspace_bytes(int Cout) {

@@ -49,6 +49,8 @@ struct IgemmParams {
   // every split writes an fp32 partial tile to y32 + split * split_stride, reduced by conv_splitk_reduce_kernel
   int splits;
   long long split_stride;
+  const float* bias;   // optional fp32 [Cout] conv bias (fprop): added to the accumulator before ReLU, the bf16 rounding
+                       // and the fused statistics; never set on split-K partials (conv_splitk_reduce_kernel adds it)
 };
 
 static constexpr int kProducerPairs = 4;
@@ -308,6 +310,11 @@ conv3d_igemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_con
         uint32_t v[32];
         tmem_ld32(t_addr + c0, v);
         tmem_ld_wait();
+        if (p.bias != nullptr) {   // warp-uniform; columns past ncol (BN = 16 x odd) re-read column 0 and are never used
+#pragma unroll
+          for (int e = 0; e < 32; ++e)
+            v[e] = __float_as_uint(__uint_as_float(v[e]) + __ldg(p.bias + n0 + c0 + (e < ncol ? e : 0)));
+        }
         if (p.stat_acc != nullptr) {   // warp-uniform branch
           float xs[32], xq[32];
 #pragma unroll
@@ -628,10 +635,10 @@ conv3d_igemm2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
   }
 }
 
-// out[v, c] = (relu)(sum_s partial[s][v][c]) -> bf16 channel window
+// out[v, c] = (relu)(sum_s partial[s][v][c] (+ bias[c])) -> bf16 channel window; the partials carry no bias
 __global__ void __launch_bounds__(256)
 conv_splitk_reduce_kernel(const float* __restrict__ partial, int splits, long long split_stride, long long NV, int C,
-                          int relu, __nv_bfloat16* __restrict__ y, int ldy, int y_coff) {
+                          int relu, __nv_bfloat16* __restrict__ y, int ldy, int y_coff, const float* __restrict__ bias) {
   pdl_prologue();
   const int C4 = C >> 2;
   const long long total = NV * C4;
@@ -644,6 +651,7 @@ conv_splitk_reduce_kernel(const float* __restrict__ partial, int splits, long lo
       const float4 t = *reinterpret_cast<const float4*>(partial + s * split_stride + v * C + c);
       a.x += t.x; a.y += t.y; a.z += t.z; a.w += t.w;
     }
+    if (bias != nullptr) { a.x += bias[c]; a.y += bias[c + 1]; a.z += bias[c + 2]; a.w += bias[c + 3]; }
     if (relu) { a.x = relu_nan(a.x); a.y = relu_nan(a.y); a.z = relu_nan(a.z); a.w = relu_nan(a.w); }
     uint2 o;
     o.x = pack_bf16x2(a.x, a.y);
@@ -674,7 +682,7 @@ static void choose_box(int W, int H, int D, int& bw, int& bh, int& bd) {
 
 bool slab_applicable(int N, int D, int H, int W, int Cin, int Cout, int y_is_fp32);
 int launch_slab(const void* x, int ldx, int x_coff, const void* wpack, void* y, int ldy, int y_coff, int N, int D,
-                int H, int W, int Cin, int Cout, int relu, long long* stat_acc, const void* stat_r,
+                int H, int W, int Cin, int Cout, int relu, long long* stat_acc, const void* stat_r, const float* bias,
                 cudaStream_t stream);
 
 int make_act_tmap(CUtensorMap* map, const void* base, int N, int D, int H, int W, int C, int ld, int coff,
@@ -708,7 +716,7 @@ using namespace b2;
 static int conv3d_igemm_impl(const void* x, int ldx, int x_coff, const void* wpack, void* y, int ldy, int y_coff,
                              int y_is_fp32, int N, int D, int H, int W, int Cin, int Cout, int relu,
                              long long* stat_acc, const void* stat_r, void* splitk_workspace,
-                             long long splitk_workspace_bytes, cudaStream_t stream) {
+                             long long splitk_workspace_bytes, const float* bias, cudaStream_t stream) {
   B2_REQUIRE(x && wpack && y, "b2_conv3d_igemm: null pointer");
   B2_REQUIRE(N > 0 && D > 0 && H > 0 && W > 0, "b2_conv3d_igemm: bad shape %dx%dx%dx%d", N, D, H, W);
   B2_REQUIRE(Cin % 16 == 0 && Cin >= 16, "b2_conv3d_igemm: Cin=%d must be a multiple of 16", Cin);
@@ -720,7 +728,8 @@ static int conv3d_igemm_impl(const void* x, int ldx, int x_coff, const void* wpa
   // narrow-N layers at (almost) tile-aligned resolutions: shared-memory tap-reuse kernel (conv_slab.cu)
   static const bool no_slab = getenv("B2_NO_SLAB") != nullptr;
   if (!no_slab && slab_applicable(N, D, H, W, Cin, Cout, y_is_fp32))
-    return launch_slab(x, ldx, x_coff, wpack, y, ldy, y_coff, N, D, H, W, Cin, Cout, relu, stat_acc, stat_r, stream);
+    return launch_slab(x, ldx, x_coff, wpack, y, ldy, y_coff, N, D, H, W, Cin, Cout, relu, stat_acc, stat_r, bias,
+                       stream);
 
   IgemmParams p;
   p.N = N; p.D = D; p.H = H; p.W = W; p.Cin = Cin; p.Cout = Cout;
@@ -771,6 +780,7 @@ static int conv3d_igemm_impl(const void* x, int ldx, int x_coff, const void* wpa
   }
   p.stat_acc = stat_acc;
   p.stat_r = reinterpret_cast<const __nv_bfloat16*>(stat_r);
+  p.bias = bias;
   if (stat_acc) {
     B2_REQUIRE(N == 1 && p.n_tiles_n == 1 && !y_is_fp32,
                "b2_conv3d_igemm_stats: fused statistics need batch 1, Cout <= 256 and a bf16 output");
@@ -788,10 +798,10 @@ static int conv3d_igemm_impl(const void* x, int ldx, int x_coff, const void* wpa
   }
   // wide layers: CTA pairs (each CTA stages half of the weight tile), see conv3d_igemm2_kernel.  Opt-in (B2_2CTA=1):
   // bit-identical results, but measured SLOWER than the one-CTA kernel on B200 in round 1
-  // (profiles/r01_bench_kernels_2cta.txt)
+  // (profiles/r01_bench_kernels_2cta.txt).  Biased launches stay on the one-CTA kernels, whose epilogue adds the bias.
   static const bool no_pairs = getenv("B2_2CTA") == nullptr;
   const long long m_tiles = p.total_tiles / p.n_tiles_n;
-  if (!no_pairs && p.KC == 64 && BN >= 128 && p.splits == 1 && !y_is_fp32 && m_tiles >= 8) {
+  if (!no_pairs && !bias && p.KC == 64 && BN >= 128 && p.splits == 1 && !y_is_fp32 && m_tiles >= 8) {
     p.b_bytes = (BN / 2) * p.KC * 2;
     p.stages = smem_budget / (p.a_bytes + p.b_bytes);
     if (p.stages > 12) p.stages = 12;
@@ -853,6 +863,7 @@ static int conv3d_igemm_impl(const void* x, int ldx, int x_coff, const void* wpa
     p.ldy = Cout;
     p.y_coff = 0;
     p.relu = 0;
+    p.bias = nullptr;
   }
   const long long work_items = p.total_tiles * p.splits;
   long long grid = work_items < num_sms() ? work_items : num_sms();
@@ -876,7 +887,7 @@ static int conv3d_igemm_impl(const void* x, int ldx, int x_coff, const void* wpa
     if (rb > num_sms() * 8) rb = num_sms() * 8;
     B2_LAUNCH(conv_splitk_reduce_kernel, (unsigned)rb, 256, 0, stream, splitk_ws, p.splits, p.split_stride, NV, Cout,
                                                                 user_relu, reinterpret_cast<__nv_bfloat16*>(y),
-                                                                user_ldy, user_coff);
+                                                                user_ldy, user_coff, bias);
     B2_CHECK_CUDA(cudaGetLastError());
   }
   return B2_OK;
@@ -887,7 +898,7 @@ extern "C" int b2_conv3d_igemm(const void* x, int ldx, int x_coff, const void* w
                                int y_is_fp32, int N, int D, int H, int W, int Cin, int Cout, int relu,
                                cudaStream_t stream) {
   return conv3d_igemm_impl(x, ldx, x_coff, wpack, y, ldy, y_coff, y_is_fp32, N, D, H, W, Cin, Cout, relu, nullptr,
-                           nullptr, nullptr, 0, stream);
+                           nullptr, nullptr, 0, nullptr, stream);
 }
 
 // Same as b2_conv3d_igemm with an optional fp32 workspace: layers with fewer than num_SMs/2 output tiles are split
@@ -899,7 +910,7 @@ extern "C" int b2_conv3d_igemm_splitk(const void* x, int ldx, int x_coff, const 
                                       int y_coff, int N, int D, int H, int W, int Cin, int Cout, int relu,
                                       void* workspace, long long workspace_bytes, cudaStream_t stream) {
   return conv3d_igemm_impl(x, ldx, x_coff, wpack, y, ldy, y_coff, 0, N, D, H, W, Cin, Cout, relu, nullptr, nullptr,
-                           workspace, workspace_bytes, stream);
+                           workspace, workspace_bytes, nullptr, stream);
 }
 
 // fprop with the GroupNorm statistics of the stored (bf16-rounded, post-ReLU) output fused into the epilogue.
@@ -910,7 +921,7 @@ extern "C" int b2_conv3d_igemm_stats(const void* x, int ldx, int x_coff, const v
                                      long long* stat_acc, cudaStream_t stream) {
   B2_REQUIRE(stat_acc, "b2_conv3d_igemm_stats: null pointer");
   return conv3d_igemm_impl(x, ldx, x_coff, wpack, y, ldy, y_coff, 0, N, D, H, W, Cin, Cout, relu, stat_acc, nullptr,
-                           nullptr, 0, stream);
+                           nullptr, 0, nullptr, stream);
 }
 
 // dgrad (x = dY, wpack = dgrad pack, output dX written densely) with the GroupNorm-BACKWARD statistics of the layer
@@ -921,5 +932,17 @@ extern "C" int b2_conv3d_igemm_bstats(const void* x, int ldx, int x_coff, const 
                                       cudaStream_t stream) {
   B2_REQUIRE(stat_acc && r, "b2_conv3d_igemm_bstats: null pointer");
   return conv3d_igemm_impl(x, ldx, x_coff, wpack, y, Cout, 0, 0, N, D, H, W, Cin, Cout, 0, stat_acc, r, nullptr, 0,
-                           stream);
+                           nullptr, stream);
+}
+
+// fprop of a layer with a conv bias (fp32 [Cout]): the bias joins the fp32 accumulator before ReLU in every path the
+// launch can take (slab, plain / h-halo implicit GEMM, the fp32 output, the split-K reduction), so the stored output and
+// the fused statistics (stat_acc, optional: batch 1, Cout <= 256) see conv + bias.  splitk_workspace is optional.
+extern "C" int b2_conv3d_igemm_bias(const void* x, int ldx, int x_coff, const void* wpack, void* y, int ldy, int y_coff,
+                                    int y_is_fp32, int N, int D, int H, int W, int Cin, int Cout, int relu,
+                                    const float* bias, long long* stat_acc, void* splitk_workspace,
+                                    long long splitk_workspace_bytes, cudaStream_t stream) {
+  B2_REQUIRE(bias && (reinterpret_cast<uintptr_t>(bias) & 7) == 0, "b2_conv3d_igemm_bias: bias must be 8-byte aligned");
+  return conv3d_igemm_impl(x, ldx, x_coff, wpack, y, ldy, y_coff, y_is_fp32, N, D, H, W, Cin, Cout, relu, stat_acc,
+                           nullptr, stat_acc ? nullptr : splitk_workspace, splitk_workspace_bytes, bias, stream);
 }

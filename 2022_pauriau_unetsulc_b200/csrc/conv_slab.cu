@@ -36,6 +36,7 @@ struct SlabParams {
   __nv_bfloat16* y;
   long long* stat_acc;   // optional [Cout][4] fixed-point statistics accumulators (see conv_igemm.cu, common.h)
   const __nv_bfloat16* stat_r;   // optional: backward statistics (sum dy, sum dy*r)
+  const float* bias;             // fp32 [Cout] conv bias of the kBias instantiation, added before ReLU
   long long total_tiles;
 };
 
@@ -45,7 +46,8 @@ static constexpr int kTD = 4;
 // kTW x kTH x kTD output tile with kTW * kTH = 128 voxels per plane: 32 x 4 (round 1) or 16 x 8 — the second shape cuts
 // the tile-quantisation waste of volumes whose W is not a multiple of 32 (bounding boxes of real cohorts: W = 72 pads to
 // 80 instead of 96).  Both keep every h-tap offset (kTW rows) a multiple of the 8-row swizzle atom.
-template <int KC, int kTW>
+// kBias: layers with a conv bias (a separate instantiation: a run-time test costs the bias-free epilogue registers).
+template <int KC, int kTW, bool kBias>
 __global__ void __launch_bounds__(kSlabThreads, 1)
 conv3d_slab_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                    const SlabParams p) {
@@ -247,6 +249,11 @@ conv3d_slab_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_cons
 #pragma unroll
         for (int e = 0; e < 16; ++e) {
           float f0 = __uint_as_float(v[2 * e]), f1 = __uint_as_float(v[2 * e + 1]);
+          if constexpr (kBias) {
+            const float2 b = __ldg(reinterpret_cast<const float2*>(p.bias + c0) + e);
+            f0 += b.x;
+            f1 += b.y;
+          }
           if (p.relu) { f0 = relu_nan(f0); f1 = relu_nan(f1); }
           pk[e] = pack_bf16x2(f0, f1);
         }
@@ -340,18 +347,25 @@ bool slab_applicable(int N, int D, int H, int W, int Cin, int Cout, int y_is_fp3
   return true;
 }
 
-template <int KC, int TW>
-static int launch_slab_t(const CUtensorMap& ta, const CUtensorMap& tb, const SlabParams& p, size_t smem_bytes,
+template <int KC, int TW, bool kBias>
+static int launch_slab_b(const CUtensorMap& ta, const CUtensorMap& tb, const SlabParams& p, size_t smem_bytes,
                          cudaStream_t stream) {
   long long grid = p.total_tiles < num_sms() ? p.total_tiles : num_sms();
-  B2_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab_kernel<KC, TW>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-  B2_LAUNCH((conv3d_slab_kernel<KC, TW>), (unsigned)grid, kSlabThreads, smem_bytes, stream, ta, tb, p);
+  B2_CHECK_CUDA(cudaFuncSetAttribute(conv3d_slab_kernel<KC, TW, kBias>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     227 * 1024));
+  B2_LAUNCH((conv3d_slab_kernel<KC, TW, kBias>), (unsigned)grid, kSlabThreads, smem_bytes, stream, ta, tb, p);
   B2_CHECK_CUDA(cudaGetLastError());
   return B2_OK;
 }
+template <int KC, int TW>
+static int launch_slab_t(const CUtensorMap& ta, const CUtensorMap& tb, const SlabParams& p, size_t smem_bytes,
+                         cudaStream_t stream) {
+  return p.bias ? launch_slab_b<KC, TW, true>(ta, tb, p, smem_bytes, stream)
+                : launch_slab_b<KC, TW, false>(ta, tb, p, smem_bytes, stream);
+}
 
 int launch_slab(const void* x, int ldx, int x_coff, const void* wpack, void* y, int ldy, int y_coff, int N, int D,
-                int H, int W, int Cin, int Cout, int relu, long long* stat_acc, const void* stat_r,
+                int H, int W, int Cin, int Cout, int relu, long long* stat_acc, const void* stat_r, const float* bias,
                 cudaStream_t stream) {
   SlabParams p;
   p.N = N; p.D = D; p.H = H; p.W = W; p.Cin = Cin; p.Cout = Cout;
@@ -367,6 +381,7 @@ int launch_slab(const void* x, int ldx, int x_coff, const void* wpack, void* y, 
   p.total_tiles = (long long)N * p.tiles_w * p.tiles_h * p.tiles_d;
   p.stat_acc = stat_acc;
   p.stat_r = reinterpret_cast<const __nv_bfloat16*>(stat_r);
+  p.bias = bias;
   if (stat_acc) B2_REQUIRE(N == 1, "b2_conv3d_igemm_stats: fused statistics need batch 1");
   const int plane_bytes = tw * (th + 2) * KC * 2;
   const int b_bytes = 9 * Cout * KC * 2;

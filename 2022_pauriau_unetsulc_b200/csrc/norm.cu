@@ -464,11 +464,16 @@ gn_bwd_stats_kernel(const __nv_bfloat16* __restrict__ dy, int lddy, int dy_coff,
   if (threadIdx.x == 0) counters[N] = 0;
 }
 
-template <bool kRowLabels>   // separate instantiation: the label test must not touch the code of the dense launches
+// kBias (layers with a conv bias): the kernel also sums the STORED (bf16-rounded) dr per channel — the bias gradient.
+// Each thread keeps fp32 running sums of its channel octet, the block combines them in thread order through shared
+// memory and commits one fixed-point atomic per channel into dbias_acc int64 [C][2] (common.h): bit-identical run to run.
+// Separate instantiations: neither the label test nor the sums touch the code of the other launches.
+template <bool kRowLabels, bool kBias>
 __global__ void __launch_bounds__(256)
 gn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dy, int lddy, int dy_coff, const __nv_bfloat16* __restrict__ r,
                     long long V, int C, const float* __restrict__ mean_rstd, const float* __restrict__ coef,
-                    __nv_bfloat16* __restrict__ dr, const long long* __restrict__ row_labels) {
+                    __nv_bfloat16* __restrict__ dr, const long long* __restrict__ row_labels,
+                    long long* __restrict__ dbias_acc) {
   pdl_prologue();
   // row_labels != NULL (gradient produced by the head kernel): dy rows of voxels with label < 0 were never written
   // and count as zero — they are not read (no memset of dy, 97 % of its rows skipped)
@@ -488,6 +493,16 @@ gn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dy, int lddy, int dy_coff,
     kb[k] = cf.y;
     kc[k] = cf.z;
   }
+  float sb[8];   // kBias: running sums of the stored dr of this thread's channel octet
+#pragma unroll
+  for (int k = 0; k < 8; ++k) sb[k] = 0.f;
+  auto add_bias_sums = [&](const uint4& stored) {
+    if constexpr (kBias) {
+      const f8 q = unpack8(stored);
+#pragma unroll
+      for (int k = 0; k < 8; ++k) sb[k] += q.v[k];
+    }
+  };
   const __nv_bfloat16* rp = r + ((size_t)n * V) * C + oct * 8;
   const __nv_bfloat16* gp = dy + ((size_t)n * V) * lddy + dy_coff + oct * 8;
   __nv_bfloat16* op = dr + ((size_t)n * V) * C + oct * 8;
@@ -510,7 +525,9 @@ gn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dy, int lddy, int dy_coff,
         const float d = fmaf(ca[k], g.v[k], fmaf(kb[k], x.v[k], kc[k]));
         o.v[k] = x.v[k] > 0.f ? d : 0.f;
       }
-      stg16(op + (v + j * vstride) * C, pack8(o));
+      const uint4 pk = pack8(o);
+      add_bias_sums(pk);
+      stg16(op + (v + j * vstride) * C, pk);
     }
   }
   for (; v + vstride < V; v += 2 * vstride) {
@@ -527,8 +544,11 @@ gn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dy, int lddy, int dy_coff,
       o0.v[k] = x0.v[k] > 0.f ? d0 : 0.f;
       o1.v[k] = x1.v[k] > 0.f ? d1 : 0.f;
     }
-    stg16(op + v * C, pack8(o0));
-    stg16(op + (v + vstride) * C, pack8(o1));
+    const uint4 pk0 = pack8(o0), pk1 = pack8(o1);
+    add_bias_sums(pk0);
+    add_bias_sums(pk1);
+    stg16(op + v * C, pk0);
+    stg16(op + (v + vstride) * C, pk1);
   }
   for (; v < V; v += vstride) {
     const bool l0 = !kRowLabels || __ldg(row_labels + (size_t)n * V + v) >= 0;
@@ -540,8 +560,29 @@ gn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dy, int lddy, int dy_coff,
       const float d = fmaf(ca[k], g.v[k], fmaf(kb[k], x.v[k], kc[k]));
       o.v[k] = x.v[k] > 0.f ? d : 0.f;
     }
-    stg16(op + v * C, pack8(o));
+    const uint4 pk = pack8(o);
+    add_bias_sums(pk);
+    stg16(op + v * C, pk);
   }
+  if constexpr (kBias) {
+    __shared__ float s_sb[256][8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) s_sb[threadIdx.x][k] = sb[k];
+    __syncthreads();
+    for (int c = threadIdx.x; c < C; c += blockDim.x) {   // threads j * C8 + c / 8 hold channel c, summed in order of j
+      float a = 0.f;
+      for (int j = 0; j < vpb; ++j) a += s_sb[j * C8 + (c >> 3)][c & 7];
+      stat_atomic_add(dbias_acc + 2 * c, a);
+    }
+  }
+}
+
+// dbias_acc int64 [C][2] -> dbias fp32 [C]
+__global__ void __launch_bounds__(kMaxAccC)
+dbias_finalize_kernel(const long long* __restrict__ dbias_acc, int C, float* __restrict__ dbias) {
+  pdl_prologue();
+  const int c = threadIdx.x;
+  if (c < C) dbias[c] = (float)stat_read(dbias_acc + 2 * c);
 }
 
 static inline int stat_blocks(long long V, int C) {
@@ -657,9 +698,10 @@ extern "C" int b2_relu_gn_bwd(const void* dy, int lddy, int dy_coff, const void*
       reinterpret_cast<const __nv_bfloat16*>(dy), lddy, dy_coff, reinterpret_cast<const __nv_bfloat16*>(r), V, C,
       mean_rstd, partial, counters, N, G, gamma, coef, dgb_n, dgamma, dbeta);
   B2_CHECK_CUDA(cudaGetLastError());
-  B2_LAUNCH(gn_bwd_apply_kernel<false>, dim3(apply_blocks(V * (C / 8)), N), 256, 0, stream, 
+  B2_LAUNCH((gn_bwd_apply_kernel<false, false>), dim3(apply_blocks(V * (C / 8)), N), 256, 0, stream, 
       reinterpret_cast<const __nv_bfloat16*>(dy), lddy, dy_coff, reinterpret_cast<const __nv_bfloat16*>(r), V, C,
-      mean_rstd, coef, reinterpret_cast<__nv_bfloat16*>(dr), static_cast<const long long*>(nullptr));
+      mean_rstd, coef, reinterpret_cast<__nv_bfloat16*>(dr), static_cast<const long long*>(nullptr),
+      static_cast<long long*>(nullptr));
   B2_CHECK_CUDA(cudaGetLastError());
   return B2_OK;
 }
@@ -688,13 +730,84 @@ extern "C" int b2_relu_gn_bwd_acc(const long long* stat_acc, const void* dy, int
             1.0 / ((double)V * (C / G)), gamma, mean_rstd, coef, dgamma, dbeta);
   B2_CHECK_CUDA(cudaGetLastError());
   if (dy_row_labels != nullptr)
-    B2_LAUNCH_DEP(gn_bwd_apply_kernel<true>, dim3(apply_blocks(V * (C / 8)), 1), 256, 0, stream,
+    B2_LAUNCH_DEP((gn_bwd_apply_kernel<true, false>), dim3(apply_blocks(V * (C / 8)), 1), 256, 0, stream,
               reinterpret_cast<const __nv_bfloat16*>(dy), lddy, dy_coff, reinterpret_cast<const __nv_bfloat16*>(r), V,
-              C, mean_rstd, static_cast<const float*>(coef), reinterpret_cast<__nv_bfloat16*>(dr), dy_row_labels);
+              C, mean_rstd, static_cast<const float*>(coef), reinterpret_cast<__nv_bfloat16*>(dr), dy_row_labels,
+              static_cast<long long*>(nullptr));
   else
-    B2_LAUNCH_DEP(gn_bwd_apply_kernel<false>, dim3(apply_blocks(V * (C / 8)), 1), 256, 0, stream,
+    B2_LAUNCH_DEP((gn_bwd_apply_kernel<false, false>), dim3(apply_blocks(V * (C / 8)), 1), 256, 0, stream,
               reinterpret_cast<const __nv_bfloat16*>(dy), lddy, dy_coff, reinterpret_cast<const __nv_bfloat16*>(r), V,
-              C, mean_rstd, static_cast<const float*>(coef), reinterpret_cast<__nv_bfloat16*>(dr), dy_row_labels);
+              C, mean_rstd, static_cast<const float*>(coef), reinterpret_cast<__nv_bfloat16*>(dr), dy_row_labels,
+              static_cast<long long*>(nullptr));
   B2_CHECK_CUDA(cudaGetLastError());
   return B2_OK;
+}
+
+// ---- layers with a conv bias: the same two GroupNorm-backward forms, also producing dbias = sum_v dr[v, c] --------------
+// dbias_acc: int64 [C][2] fixed-point accumulators, zero before the call; dbias: fp32 [C] (overwritten).  The sums are
+// fused into the apply pass (gn_bwd_apply_kernel<.., true>); one more one-block launch converts them to fp32.
+static int launch_dbias_apply(const void* dy, int lddy, int dy_coff, const void* r, int N, long long V, int C,
+                              const float* mean_rstd, const float* coef, void* dr, const long long* dy_row_labels,
+                              long long* dbias_acc, float* dbias, cudaStream_t stream) {
+  const dim3 grid(apply_blocks(V * (C / 8)), N);
+  auto* dyb = reinterpret_cast<const __nv_bfloat16*>(dy);
+  auto* rb = reinterpret_cast<const __nv_bfloat16*>(r);
+  auto* drb = reinterpret_cast<__nv_bfloat16*>(dr);
+  if (dy_row_labels != nullptr)
+    B2_LAUNCH((gn_bwd_apply_kernel<true, true>), grid, 256, 0, stream, dyb, lddy, dy_coff, rb, V, C, mean_rstd, coef,
+              drb, dy_row_labels, dbias_acc);
+  else
+    B2_LAUNCH((gn_bwd_apply_kernel<false, true>), grid, 256, 0, stream, dyb, lddy, dy_coff, rb, V, C, mean_rstd, coef,
+              drb, dy_row_labels, dbias_acc);
+  B2_CHECK_CUDA(cudaGetLastError());
+  B2_LAUNCH(dbias_finalize_kernel, 1, (C + 31) / 32 * 32, 0, stream, static_cast<const long long*>(dbias_acc), C,
+            dbias);
+  B2_CHECK_CUDA(cudaGetLastError());
+  return B2_OK;
+}
+
+extern "C" int b2_relu_gn_bwd_dbias(const void* dy, int lddy, int dy_coff, const void* r, int N, long long V, int C,
+                                    int G, const float* gamma, const float* mean_rstd, void* dr, float* dgamma,
+                                    float* dbeta, void* workspace, long long workspace_bytes, int* counters,
+                                    long long* dbias_acc, float* dbias, cudaStream_t stream) {
+  B2_REQUIRE(dy && r && gamma && mean_rstd && dr && workspace && counters && dbias_acc && dbias,
+             "b2_relu_gn_bwd_dbias: null pointer");
+  int rc = check_gn_shape("b2_relu_gn_bwd_dbias", N, V, C, G);
+  if (rc) return rc;
+  B2_REQUIRE(C <= kMaxAccC, "b2_relu_gn_bwd_dbias: C=%d > %d", C, kMaxAccC);
+  B2_REQUIRE(lddy % 8 == 0 && dy_coff % 8 == 0, "b2_relu_gn_bwd_dbias: lddy/dy_coff must be multiples of 8");
+  const long long need = b2_relu_gn_bwd_workspace_bytes(N, C);
+  B2_REQUIRE(workspace_bytes >= need, "b2_relu_gn_bwd_dbias: workspace %lld < %lld", workspace_bytes, need);
+  float* partial = reinterpret_cast<float*>(workspace);
+  float* coef = partial + (size_t)N * kStatBlocks * C * 2;
+  float* dgb_n = coef + (size_t)N * C * 4;
+  const int nblk = stat_blocks(V, C);
+  const int vpi = kStatThreads / (C / 8);
+  const size_t sh = (size_t)vpi * C * 2 * sizeof(float);
+  B2_LAUNCH(gn_bwd_stats_kernel, dim3(nblk, N), kStatThreads, sh, stream,
+      reinterpret_cast<const __nv_bfloat16*>(dy), lddy, dy_coff, reinterpret_cast<const __nv_bfloat16*>(r), V, C,
+      mean_rstd, partial, counters, N, G, gamma, coef, dgb_n, dgamma, dbeta);
+  B2_CHECK_CUDA(cudaGetLastError());
+  return launch_dbias_apply(dy, lddy, dy_coff, r, N, V, C, mean_rstd, coef, dr, nullptr, dbias_acc, dbias, stream);
+}
+
+extern "C" int b2_relu_gn_bwd_acc_dbias(const long long* stat_acc, const void* dy, int lddy, int dy_coff, const void* r,
+                                        long long V, int C, int G, const float* gamma, const float* mean_rstd, void* dr,
+                                        float* dgamma, float* dbeta, void* workspace, long long workspace_bytes,
+                                        const long long* dy_row_labels, long long* dbias_acc, float* dbias,
+                                        cudaStream_t stream) {
+  B2_REQUIRE(stat_acc && dy && r && gamma && mean_rstd && dr && workspace && dbias_acc && dbias,
+             "b2_relu_gn_bwd_acc_dbias: null pointer");
+  int rc = check_gn_shape("b2_relu_gn_bwd_acc_dbias", 1, V, C, G);
+  if (rc) return rc;
+  B2_REQUIRE(C <= kMaxAccC, "b2_relu_gn_bwd_acc_dbias: C=%d > %d", C, kMaxAccC);
+  B2_REQUIRE(lddy % 8 == 0 && dy_coff % 8 == 0, "b2_relu_gn_bwd_acc_dbias: lddy/dy_coff must be multiples of 8");
+  B2_REQUIRE(workspace_bytes >= (long long)C * 4 * (long long)sizeof(float),
+             "b2_relu_gn_bwd_acc_dbias: workspace too small");
+  float* coef = reinterpret_cast<float*>(workspace);
+  B2_LAUNCH_DEP(gn_bwd_finalize_acc_kernel, 1, (C + 31) / 32 * 32, 0, stream, stat_acc, C, G,
+            1.0 / ((double)V * (C / G)), gamma, mean_rstd, coef, dgamma, dbeta);
+  B2_CHECK_CUDA(cudaGetLastError());
+  return launch_dbias_apply(dy, lddy, dy_coff, r, 1, V, C, mean_rstd, coef, dr, dy_row_labels, dbias_acc, dbias,
+                            stream);
 }

@@ -29,7 +29,7 @@ GN_EPS = 1e-5
 #            (its blocks delay CTAs of the persistent 148-CTA convolution grids; removed)
 _WGRAD_REDUCE = os.environ.get("B2_WGRAD_REDUCE", "inline")
 
-def _double_conv(in_ch, out_ch, encoder, order, num_groups):
+def _double_conv(in_ch, out_ch, encoder, order, num_groups, conv_bias=False):
     if encoder:
         c1 = (in_ch, max(out_ch // 2, in_ch))
         c2 = (c1[1], out_ch)
@@ -38,7 +38,7 @@ def _double_conv(in_ch, out_ch, encoder, order, num_groups):
         c2 = (out_ch, out_ch)
     seq = nn.Sequential()
     for pos, (ci, co) in ((1, c1), (2, c2)):
-        seq.add_module("conv%d" % pos, nn.Conv3d(ci, co, 3, padding=1, bias=False))
+        seq.add_module("conv%d" % pos, nn.Conv3d(ci, co, 3, padding=1, bias=conv_bias))
         seq.add_module("relu%d" % pos, nn.ReLU())
         seq.add_module("norm%d" % pos, nn.GroupNorm(num_groups, co, eps=GN_EPS))
     return seq
@@ -47,10 +47,10 @@ def _double_conv(in_ch, out_ch, encoder, order, num_groups):
 class _Block(nn.Module):
     """Parameter holder for one encoder / decoder level (names match upstream: ``double_conv.conv1`` ...)."""
 
-    def __init__(self, in_ch, out_ch, encoder, order, num_groups, is_max_pool=False):
+    def __init__(self, in_ch, out_ch, encoder, order, num_groups, is_max_pool=False, conv_bias=False):
         super().__init__()
         self.is_max_pool = is_max_pool
-        self.double_conv = _double_conv(in_ch, out_ch, encoder, order, num_groups)
+        self.double_conv = _double_conv(in_ch, out_ch, encoder, order, num_groups, conv_bias)
 
     def forward(self, *a, **k):  # never used: the network is executed by UNet3D as a whole
         raise RuntimeError("unetsulc_b200 blocks are parameter holders; call UNet3D.forward")
@@ -85,8 +85,11 @@ class _Saved(object):
 
 
 class UNet3D(nn.Module):
+    """conv_bias: the 14 trunk convolutions carry a bias (the 58-key checkpoint layout of the 2018 pytorch-3dunet
+    ``DoubleConv``, ``nn.Conv3d(..., padding=1)``).  ``load_state_dict`` switches the layout to the checkpoint's."""
+
     def __init__(self, in_channels, out_channels, final_sigmoid=False, interpolate=True, dropout=0.,
-                 conv_layer_order='crg', init_channel_number=64):
+                 conv_layer_order='crg', init_channel_number=64, conv_bias=False):
         super().__init__()
         if in_channels != 1:
             raise ValueError("unetsulc_b200.UNet3D: in_channels=%r unsupported (skeleton volumes have 1)" % in_channels)
@@ -107,15 +110,16 @@ class UNet3D(nn.Module):
         self.num_groups = g
         self.init_channel_number = f
         o = conv_layer_order
+        cb = bool(conv_bias)
         self.encoders = nn.ModuleList([
-            _Block(in_channels, f, True, o, g, False),
-            _Block(f, 2 * f, True, o, g, True),
-            _Block(2 * f, 4 * f, True, o, g, True),
-            _Block(4 * f, 8 * f, True, o, g, True)])
+            _Block(in_channels, f, True, o, g, False, cb),
+            _Block(f, 2 * f, True, o, g, True, cb),
+            _Block(2 * f, 4 * f, True, o, g, True, cb),
+            _Block(4 * f, 8 * f, True, o, g, True, cb)])
         self.decoders = nn.ModuleList([
-            _Block(4 * f + 8 * f, 4 * f, False, o, g),
-            _Block(2 * f + 4 * f, 2 * f, False, o, g),
-            _Block(f + 2 * f, f, False, o, g)])
+            _Block(4 * f + 8 * f, 4 * f, False, o, g, conv_bias=cb),
+            _Block(2 * f + 4 * f, 2 * f, False, o, g, conv_bias=cb),
+            _Block(f + 2 * f, f, False, o, g, conv_bias=cb)])
         self.final_conv = nn.Conv3d(f, out_channels, 1)
         self.final_activation = nn.Softmax(dim=1)
         self._layers_cache = None
@@ -189,11 +193,51 @@ class UNet3D(nn.Module):
             b = Wk @ b + m.bias
         return W.reshape(W.shape[0], W.shape[1], 1, 1, 1), b
 
+    # ------------------------------------------------------------------------------------------ conv-bias layout
+    def _trunk_convs(self):
+        return [getattr(blk.double_conv, "conv%d" % k) for blk in list(self.encoders) + list(self.decoders)
+                for k in (1, 2)]
+
+    @property
+    def conv_bias(self):
+        """True when the 14 trunk convolutions carry a bias (58-key layout), False for the 44-key layout"""
+        return self.encoders[0].double_conv.conv1.bias is not None
+
+    def trunk_stride(self):
+        """trunk parameters per conv layer in trunk_parameters(): 3 (w, gamma, beta) or 4 (w, b, gamma, beta)"""
+        return 4 if self.conv_bias else 3
+
+    def set_conv_bias(self, flag):
+        """Switch the trunk between the bias-free and the biased layout.  New biases are zero Parameters on the conv
+        weight's device and dtype.  Cached layer lists and statistics pools are rebuilt; an optimiser built before
+        the switch does not see the new parameters (build it afterwards, as every training flow here does)."""
+        flag = bool(flag)
+        if flag == self.conv_bias:
+            return
+        for conv in self._trunk_convs():
+            w = conv.weight
+            conv.bias = nn.Parameter(torch.zeros(conv.out_channels, device=w.device, dtype=w.dtype)) if flag else None
+        self._layers_cache = None
+        self.__dict__.pop("_stat_pool", None)
+
+    def load_state_dict(self, state_dict, strict=True, assign=False):
+        """Follows the checkpoint's layout: with all 14 ``double_conv.conv{1,2}.bias`` keys the model becomes biased,
+        with none of them bias-free; a partial set is an error naming the missing keys."""
+        names = ["%s.%d.double_conv.conv%d.bias" % (part, j, k)
+                 for part, n in (("encoders", 4), ("decoders", 3)) for j in range(n) for k in (1, 2)]
+        have = [k for k in names if k in state_dict]
+        if have and len(have) != len(names):
+            raise RuntimeError("unetsulc_b200.UNet3D: checkpoint has %d of the 14 trunk conv biases; missing: %s"
+                               % (len(have), ", ".join(k for k in names if k not in state_dict)))
+        self.set_conv_bias(bool(have))
+        return super().load_state_dict(state_dict, strict=strict, assign=assign)
+
     def trunk_parameters(self):
-        """Parameters in the order the autograd functions take them (14 x (w, gamma, beta))."""
+        """Parameters in the order the autograd functions take them: 14 x (w, gamma, beta), or 14 x (w, b, gamma,
+        beta) with conv biases (trunk_stride())."""
         ps = []
         for l in self._layers():
-            ps += [l.conv.weight, l.norm.weight, l.norm.bias]
+            ps += [l.conv.weight] + ([l.conv.bias] if l.conv.bias is not None else []) + [l.norm.weight, l.norm.bias]
         return ps
 
     def _check_input(self, x):
@@ -239,18 +283,35 @@ class UNet3D(nn.Module):
         pool = None
         if B == 1:                                 # statistics accumulators of this step, zeroed with one fill
             pool = self.__dict__.get("_stat_pool")
-            if pool is None or pool.buf.device != dev:
-                pool = self.__dict__["_stat_pool"] = ops.StatPool(dev)
+            if pool is None or pool.buf.device != dev:   # biased layers also take one dbias slot each in backward
+                pool = self.__dict__["_stat_pool"] = ops.StatPool(dev, 48) if self.conv_bias else ops.StatPool(dev)
             pool.reset()
 
         deferred = []
+
+        def conv_gn_bias(layer, xin, r, first, gamma, beta):
+            """the conv + bias + ReLU of a biased layer into r, with the GroupNorm statistics fused where the
+            bias-free layer fuses them; returns (mean_rstd, scale_shift)"""
+            cin, cout = layer.cin, layer.cout
+            b = layer.conv.bias.detach()
+            fuse = B == 1 and (first or (cout <= 256 and B * r.V > ops.SPLITK_MAX_VOXELS))
+            acc = ops._acc(pool, cout, dev) if fuse else None
+            if first:
+                ops.conv3d_first_fwd_bias(xin, layer.conv.weight.detach(), b, r, stat_acc=acc)
+            else:
+                ops.conv3d_igemm_bias(xin, layer.packs()[0], b, r, cin, cout, stat_acc=acc, splitk=True)
+            if fuse:
+                return ops.gn_finalize_acc(acc, r.V, cout, G, layer.norm.eps, gamma, beta)
+            return ops.relu_gn_stats(r, G, layer.norm.eps, gamma, beta)
 
         def conv_gn(layer, xin, out_view, pooled=None, first=False, defer=False):
             cin, cout = layer.cin, layer.cout
             d, h, w = (out_view.D, out_view.H, out_view.W)
             r = ActView.alloc(B, d, h, w, cout, dev)
             gamma, beta = layer.norm.weight.detach(), layer.norm.bias.detach()
-            if first and B == 1:
+            if layer.conv.bias is not None:
+                mr, ss = conv_gn_bias(layer, xin, r, first, gamma, beta)
+            elif first and B == 1:
                 mr, ss = ops.conv3d_first_fwd_gn_stats(xin, layer.conv.weight.detach(), r, G, layer.norm.eps, gamma,
                                                        beta, pool)
             elif first:
@@ -308,24 +369,26 @@ class UNet3D(nn.Module):
 
     # ------------------------------------------------------------------------------------------ trunk backward
     def _trunk_backward(self, save, dfeat, needs, outs=None, dfeat_stats=None, dfeat_row_labels=None):
-        """dfeat: ActView gradient w.r.t. the trunk output.  needs: list of 42 bools (w, gamma, beta per layer).
-        outs: optional list of 42 pre-allocated fp32 tensors the gradients are written into (views of the
-        data-parallel buckets).  Returns list of 42 grads (None where not needed)."""
+        """dfeat: ActView gradient w.r.t. the trunk output.  needs: list of 14 x trunk_stride() bools (w, [b,] gamma,
+        beta per layer).  outs: optional list of as many pre-allocated fp32 tensors the gradients are written into
+        (views of the data-parallel buckets).  Returns the list of gradients (None where not needed)."""
         L = self._layers()
         G = self.num_groups
         rec, cats, dims = save.rec, save.cats, save.dims
         skip_c, up_c = save.skip_c, save.up_c
-        grads = [None] * 42
+        S = self.trunk_stride()
+        iw, ib, ig, ibt = 0, (1 if S == 4 else None), S - 2, S - 1   # offsets of w, b, gamma, beta within a layer
+        grads = [None] * (14 * S)
         first_needed = None
         for i in range(14):
-            if needs[3 * i] or needs[3 * i + 1] or needs[3 * i + 2]:
+            if any(needs[S * i:S * i + S]):   # a layer whose only trainable parameter is its bias still needs dr
                 first_needed = i
                 break
         if first_needed is None:
             return grads
         hook = self.grad_ready_hook
         if outs is None:
-            outs = [None] * 42
+            outs = [None] * (14 * S)
 
         B = save.x.shape[0]
         # Weight gradients: the split reductions of the layers are deferred and run as ONE launch (b2_wgrad_reduce_multi)
@@ -339,7 +402,7 @@ class UNet3D(nn.Module):
             del pending[:]
             if hook is not None:
                 for j in waiting:
-                    hook(j, [g for g in grads[3 * j:3 * j + 3] if g is not None])
+                    hook(j, [g for g in grads[S * j:S * j + S] if g is not None])
             del waiting[:]
 
         def layer_bwd(i, dy, dy_stats=None):
@@ -347,26 +410,37 @@ class UNet3D(nn.Module):
             dgrad that produced it fused them).  Returns gradient w.r.t. the layer input (or None); for the second
             conv of a block the return value is (dx, stats) so that the first conv's GroupNorm skips its pass."""
             layer, rc = L[i], rec[i]
-            want_gb = needs[3 * i + 1] or needs[3 * i + 2]
-            go, bo = (outs[3 * i + 1] if want_gb else None), (outs[3 * i + 2] if want_gb else None)
-            if dy_stats is not None:
+            o = S * i
+            want_gb = needs[o + ig] or needs[o + ibt]
+            go, bo = (outs[o + ig] if want_gb else None), (outs[o + ibt] if want_gb else None)
+            labels13 = dfeat_row_labels if i == 13 else None
+            if ib is not None and needs[o + ib]:   # conv-bias gradient fused into the GroupNorm-backward apply pass
+                if dy_stats is not None:
+                    dr, dg, db, dbias = ops.relu_gn_bwd_from_stats_dbias(
+                        dy_stats, dy, rc["r"], G, layer.norm.weight.detach(), rc["mr"], want_gb, go, bo,
+                        dy_row_labels=labels13, dbias_out=outs[o + ib], pool=save.pool)
+                else:
+                    dr, dg, db, dbias = ops.relu_gn_bwd_dbias(dy, rc["r"], G, layer.norm.weight.detach(), rc["mr"],
+                                                              want_gb, go, bo, dbias_out=outs[o + ib])
+                grads[o + ib] = dbias
+            elif dy_stats is not None:
                 dr, dg, db = ops.relu_gn_bwd_from_stats(dy_stats, dy, rc["r"], G, layer.norm.weight.detach(),
                                                         rc["mr"], want_gb, go, bo,
-                                                        dy_row_labels=dfeat_row_labels if i == 13 else None)
+                                                        dy_row_labels=labels13)
             else:
                 dr, dg, db = ops.relu_gn_bwd(dy, rc["r"], G, layer.norm.weight.detach(), rc["mr"], want_gb, go, bo)
-            if needs[3 * i + 1]:
-                grads[3 * i + 1] = dg
-            if needs[3 * i + 2]:
-                grads[3 * i + 2] = db
-            if needs[3 * i]:
+            if needs[o + ig]:
+                grads[o + ig] = dg
+            if needs[o + ibt]:
+                grads[o + ibt] = db
+            if needs[o + iw]:
                 if layer.cin == 1:
-                    grads[3 * i] = ops.conv3d_first_wgrad(rc["x"], dr, layer.cout, outs[3 * i])
+                    grads[o + iw] = ops.conv3d_first_wgrad(rc["x"], dr, layer.cout, outs[o + iw])
                 elif _WGRAD_REDUCE == "inline":
-                    grads[3 * i] = ops.conv3d_wgrad(rc["x"], dr, layer.cin, layer.cout, outs[3 * i])
+                    grads[o + iw] = ops.conv3d_wgrad(rc["x"], dr, layer.cin, layer.cout, outs[o + iw])
                 else:   # "defer"
-                    desc = ops.conv3d_wgrad_partial(rc["x"], dr, layer.cin, layer.cout, i, outs[3 * i])
-                    grads[3 * i] = desc["dw"]
+                    desc = ops.conv3d_wgrad_partial(rc["x"], dr, layer.cin, layer.cout, i, outs[o + iw])
+                    grads[o + iw] = desc["dw"]
                     pending.append(desc)
             waiting.append(i)
             if hook is not None and (flush_at is None or i in flush_at):
@@ -466,14 +540,15 @@ class UNet3D(nn.Module):
 
     def forward_backward(self, x, labels, outs=None, loss_scale=1.0):
         """One fused training step without autograd: forward, CrossEntropyLoss(ignore_index=-1), backward.
-        Gradients are returned (and written into `outs`, 44 tensors in ``parameters()`` order, when given) for the
-        parameters with ``requires_grad``; nothing is accumulated into ``.grad``.
+        Gradients are returned (and written into `outs`, one tensor per ``ordered_parameters()`` entry, when given)
+        for the parameters with ``requires_grad``; nothing is accumulated into ``.grad``.
         Returns (loss_and_count: fp32 [2] = (mean, sum) device tensor, count int32 [1], preds int32 [B,D,H,W],
-        grads: list of 44 tensors or None)."""
+        grads: list of tensors or None in ordered_parameters() order)."""
         x = self._check_input(x)
         hp = self.head_parameters()
         chain = len(hp) > 2
         params = list(self.trunk_parameters()) + hp
+        nt = 14 * self.trunk_stride()
         needs = [bool(p.requires_grad) for p in params]
         if outs is None:
             outs = [None] * len(params)
@@ -485,11 +560,11 @@ class UNet3D(nn.Module):
         save = _Saved()
         with torch.no_grad():
             feat, xss = self._split_feat(self._trunk_forward(x, save, defer_last_apply=True))
-            fuse13 = x.shape[0] == 1 and any(needs[:42])
+            fuse13 = x.shape[0] == 1 and any(needs[:nt])
             out = ops.head_ce(feat, labels, hw.detach(), hb.detach(), compute_grad=True,
                               eval_softmax=False, grad_scale=float(loss_scale), want_preds=True,
-                              want_dx=any(needs[:42]), dW_out=None if chain else outs[42],
-                              db_out=None if chain else outs[43],
+                              want_dx=any(needs[:nt]), dW_out=None if chain else outs[nt],
+                              db_out=None if chain else outs[nt + 1],
                               stat_r=save.rec[13]["r"] if fuse13 else None, pool=save.pool, x_scale_shift=xss,
                               sparse_dx=fuse13)
             if self.post_head_hook is not None:    # CUDA-graph capture: segment boundary once the loss is final
@@ -502,22 +577,23 @@ class UNet3D(nn.Module):
                                          allow_unused=True)
                 for i, g in zip(live, gs):
                     g = torch.zeros_like(hp[i]) if g is None else g
-                    if outs[42 + i] is not None:
-                        outs[42 + i].copy_(g)
-                        g = outs[42 + i]
+                    if outs[nt + i] is not None:
+                        outs[nt + i].copy_(g)
+                        g = outs[nt + i]
                     head_grads[i] = g
         else:
-            head_grads = [out["dW"] if needs[42] else None, out["db"] if needs[43] else None]
+            head_grads = [out["dW"] if needs[nt] else None, out["db"] if needs[nt + 1] else None]
         with torch.no_grad():
             if self.grad_ready_hook is not None:
                 self.grad_ready_hook(14, [g for g in head_grads if g is not None])
-            grads = (self._trunk_backward(save, out["dx"], needs[:42], outs[:42], out["dx_stats"],
+            grads = (self._trunk_backward(save, out["dx"], needs[:nt], outs[:nt], out["dx_stats"],
                                           out["dx_row_labels"])
-                     if any(needs[:42]) else [None] * 42)
+                     if any(needs[:nt]) else [None] * nt)
         return out["loss"], out["count"], out["preds"], list(grads) + head_grads
 
     def ordered_parameters(self):
-        """The parameters in the order forward_backward() reports gradients (42 trunk + 2 per head conv)."""
+        """The parameters in the order forward_backward() reports gradients (14 x trunk_stride() trunk + 2 per head
+        conv: 44 or 58 with a one-conv head)."""
         return list(self.trunk_parameters()) + self.head_parameters()
 
     def scores_at(self, x, index, exact=False):
@@ -580,7 +656,10 @@ def _exact_methods():
 
         def conv_gn(i, xs, cin3, out, ld, off):
             layer = L[i]
-            r = ops.exact_conv(xs, packs[i], cin3, layer.cout, relu=True)
+            if layer.conv.bias is not None:
+                r = ops.exact_conv_bias(xs, packs[i], layer.conv.bias.detach().float(), cin3, layer.cout, relu=True)
+            else:
+                r = ops.exact_conv(xs, packs[i], cin3, layer.cout, relu=True)
             ops.exact_gn(r, G, layer.norm.eps, layer.norm.weight.detach().float(), layer.norm.bias.detach().float(),
                          out, ld, off)
 
@@ -630,16 +709,13 @@ def _exact_methods():
 UNet3D._exact_packs, UNet3D._exact_trunk, UNet3D._exact_scores_at = _exact_methods()
 
 
-def _needs(ctx_needs, offset):
-    return list(ctx_needs[offset:offset + 42])
-
-
 class _DenseFunction(torch.autograd.Function):
     @staticmethod
     def forward(ctx, model, x, softmax, *params):
         save = _Saved()
         feat = model._trunk_forward(x, save)
-        hw, hb = params[42].detach(), params[43].detach()
+        nt = len(params) - 2
+        hw, hb = params[nt].detach(), params[nt + 1].detach()
         out = ops.head_dense_fwd(feat, hw, hb, softmax=softmax)
         ctx.model, ctx.save_, ctx.feat, ctx.softmax, ctx.hw = model, save, feat, softmax, hw
         if softmax:
@@ -654,9 +730,10 @@ class _DenseFunction(torch.autograd.Function):
             (p,) = ctx.saved_tensors
             g = p * (g - (g * p).sum(dim=1, keepdim=True))
         dfeat, dW, db = ops.head_dense_bwd(g, feat, ctx.hw)
-        needs = list(ctx.needs_input_grad[3:3 + 42])
+        nt = len(ctx.needs_input_grad) - 5
+        needs = list(ctx.needs_input_grad[3:3 + nt])
         grads = model._trunk_backward(save, dfeat, needs)
-        nh = ctx.needs_input_grad[45:47]
+        nh = ctx.needs_input_grad[3 + nt:5 + nt]
         if model.grad_ready_hook is not None:
             model.grad_ready_hook(14, [t for t, n in zip((dW, db), nh) if n])
         return (None, None, None) + tuple(grads) + (dW if nh[0] else None, db if nh[1] else None)
@@ -667,7 +744,8 @@ class _FusedLossFunction(torch.autograd.Function):
     def forward(ctx, model, x, labels, *params):
         save = _Saved()
         feat = model._trunk_forward(x, save)
-        hw, hb = params[42].detach(), params[43].detach()
+        nt = len(params) - 2
+        hw, hb = params[nt].detach(), params[nt + 1].detach()
         out = ops.head_ce(feat, labels, hw, hb, compute_grad=False, eval_softmax=False)
         ctx.model, ctx.save_, ctx.feat, ctx.labels, ctx.hw, ctx.hb = model, save, feat, labels, hw, hb
         ctx.mark_non_differentiable(out["preds"])
@@ -677,12 +755,13 @@ class _FusedLossFunction(torch.autograd.Function):
     def backward(ctx, gloss, _gpreds):
         model, save, feat = ctx.model, ctx.save_, ctx.feat
         gl = gloss.detach().float().reshape(1).contiguous()
-        needs = list(ctx.needs_input_grad[3:3 + 42])
-        nh = ctx.needs_input_grad[45:47]
+        nt = len(ctx.needs_input_grad) - 5
+        needs = list(ctx.needs_input_grad[3:3 + nt])
+        nh = ctx.needs_input_grad[3 + nt:5 + nt]
         out = ops.head_ce(feat, ctx.labels, ctx.hw, ctx.hb, compute_grad=True,
                           eval_softmax=False, grad_scale=1.0, grad_scale_dev=gl, want_preds=False,
                           want_dx=any(needs))
         if model.grad_ready_hook is not None:
             model.grad_ready_hook(14, [t for t, n in zip((out["dW"], out["db"]), nh) if n])
-        grads = model._trunk_backward(save, out["dx"], needs) if any(needs) else [None] * 42
+        grads = model._trunk_backward(save, out["dx"], needs) if any(needs) else [None] * nt
         return (None, None, None) + tuple(grads) + (out["dW"] if nh[0] else None, out["db"] if nh[1] else None)

@@ -229,6 +229,81 @@ def relu_gn_bwd_from_stats(acc, dy, r, groups, gamma, mean_rstd, want_param_grad
     return dr, dgamma, dbeta
 
 
+# ---- layers with a conv bias (58-key checkpoints); the bias-free layers never call these ----------------------------
+def conv3d_igemm_bias(x, wpack, bias, y, cin, cout, relu=True, y_fp32=False, stat_acc=None, splitk=False):
+    """fprop of a biased layer: bias fp32 [cout] is added to the accumulator before ReLU.  stat_acc: fixed-point
+    statistics accumulators (batch 1, see conv3d_igemm_gn_stats); splitk: allow the split-K path on tiny volumes."""
+    lib = _lib.load()
+    _need_cuda(x.buf, wpack, y.buf, bias)
+    if not bias.is_contiguous() or bias.data_ptr() % 8:
+        bias = bias.contiguous().clone()
+    ws = None
+    if splitk and stat_acc is None and not y_fp32 and x.N * x.V <= SPLITK_MAX_VOXELS:
+        ws = Workspace.get(lib.b2_conv3d_splitk_workspace_bytes(x.N, x.D, x.H, x.W, cout), x.buf.device, "splitk")
+    with _Prof("conv3d_igemm", 2.0 * x.N * x.V * 27 * cin * cout):
+        _lib.check(lib.b2_conv3d_igemm_bias(_p(x.buf), x.ld, x.coff, _p(wpack), _p(y.buf), y.ld, y.coff, int(y_fp32),
+                                            x.N, x.D, x.H, x.W, cin, cout, int(relu), _p(bias), _p(stat_acc), _p(ws),
+                                            ws.numel() if ws is not None else 0, _s()), "b2_conv3d_igemm_bias")
+    _count(2 if ws is not None else 1)
+
+
+def conv3d_first_fwd_bias(x, w, bias, y, relu=True, stat_acc=None):
+    """first conv (Cin = 1) + bias + ReLU; stat_acc: fused GroupNorm statistics (batch 1)"""
+    lib = _lib.load()
+    _need_cuda(x, w, bias, y.buf)
+    _lib.check(lib.b2_conv3d_first_fwd_bias(_p(x), _p(w), _p(bias), _p(y.buf), y.ld, y.coff, y.N, y.D, y.H, y.W,
+                                            w.shape[0], int(relu), _p(stat_acc), _s()), "b2_conv3d_first_fwd_bias")
+    _count(1)
+
+
+def _dbias_acc(pool, C, device):
+    """int64 [C][2] zeroed dbias accumulators (half of a StatPool slot)"""
+    return (pool.take(C) if pool is not None else torch.zeros(4 * C, dtype=torch.int64, device=device))[:2 * C]
+
+
+def relu_gn_bwd_from_stats_dbias(acc, dy, r, groups, gamma, mean_rstd, want_param_grads=True, dgamma_out=None,
+                                 dbeta_out=None, dy_row_labels=None, dbias_out=None, pool=None):
+    """relu_gn_bwd_from_stats that also returns the conv-bias gradient sum_v dr (fp32 [C], into dbias_out if given).
+    Returns (dr, dgamma, dbeta, dbias)."""
+    lib = _lib.load()
+    dev = r.buf.device
+    dr = ActView.alloc(r.N, r.D, r.H, r.W, r.C, dev)
+    dgamma = dgamma_out if dgamma_out is not None else (
+        torch.empty(r.C, dtype=torch.float32, device=dev) if want_param_grads else None)
+    dbeta = dbeta_out if dbeta_out is not None else (
+        torch.empty(r.C, dtype=torch.float32, device=dev) if want_param_grads else None)
+    dbias = dbias_out if dbias_out is not None else torch.empty(r.C, dtype=torch.float32, device=dev)
+    dacc = _dbias_acc(pool, r.C, dev)
+    ws = Workspace.get(r.C * 16, dev, "gncoef")
+    _lib.check(lib.b2_relu_gn_bwd_acc_dbias(_p(acc), _p(dy.buf), dy.ld, dy.coff, _p(r.buf), r.V, r.C, groups,
+                                            _p(gamma), _p(mean_rstd), _p(dr.buf), _p(dgamma), _p(dbeta), _p(ws),
+                                            ws.numel(), _p(dy_row_labels), _p(dacc), _p(dbias), _s()),
+               "b2_relu_gn_bwd_acc_dbias")
+    _count(3)
+    return dr, dgamma, dbeta, dbias
+
+
+def relu_gn_bwd_dbias(dy, r, groups, gamma, mean_rstd, want_param_grads=True, dgamma_out=None, dbeta_out=None,
+                      dbias_out=None):
+    """relu_gn_bwd that also returns the conv-bias gradient (summed over the samples).  Returns (dr, dgamma, dbeta,
+    dbias)."""
+    lib = _lib.load()
+    dev = r.buf.device
+    dr = ActView.alloc(r.N, r.D, r.H, r.W, r.C, dev)
+    dgamma = dgamma_out if dgamma_out is not None else (
+        torch.empty(r.C, dtype=torch.float32, device=dev) if want_param_grads else None)
+    dbeta = dbeta_out if dbeta_out is not None else (
+        torch.empty(r.C, dtype=torch.float32, device=dev) if want_param_grads else None)
+    dbias = dbias_out if dbias_out is not None else torch.empty(r.C, dtype=torch.float32, device=dev)
+    dacc = _dbias_acc(None, r.C, dev)
+    ws = Workspace.get(lib.b2_relu_gn_bwd_workspace_bytes(r.N, r.C), dev, "gn")
+    _lib.check(lib.b2_relu_gn_bwd_dbias(_p(dy.buf), dy.ld, dy.coff, _p(r.buf), r.N, r.V, r.C, groups, _p(gamma),
+                                        _p(mean_rstd), _p(dr.buf), _p(dgamma), _p(dbeta), _p(ws), ws.numel(),
+                                        _p(_counters(dev)), _p(dacc), _p(dbias), _s()), "b2_relu_gn_bwd_dbias")
+    _count(4)   # zero fill of the accumulators, statistics, apply, dbias finalize
+    return dr, dgamma, dbeta, dbias
+
+
 def conv3d_wgrad(x, dy, cin, cout, out=None):
     """returns dW fp32 [cout, cin, 3, 3, 3] (written into `out` when given)"""
     lib = _lib.load()
@@ -737,6 +812,15 @@ def exact_conv(xsplit, wpack, cin3, cout, relu=True):
     r = torch.empty((xsplit.V, cout), dtype=F32, device=dev)
     y = ActView(r, 1, xsplit.D, xsplit.H, xsplit.W, cout)
     conv3d_igemm(xsplit, wpack, y, cin3, cout, relu=relu, y_fp32=True)
+    return r
+
+
+def exact_conv_bias(xsplit, wpack, bias, cin3, cout, relu=True):
+    """exact_conv of a biased layer: the fp32 bias joins the fp32 accumulator before ReLU"""
+    dev = xsplit.buf.device
+    r = torch.empty((xsplit.V, cout), dtype=F32, device=dev)
+    y = ActView(r, 1, xsplit.D, xsplit.H, xsplit.W, cout)
+    conv3d_igemm_bias(xsplit, wpack, bias, y, cin3, cout, relu=relu, y_fp32=True)
     return r
 
 

@@ -1,4 +1,4 @@
-"""Fused multi-tensor SGD (one launch of sgd_multi_kernel for all 44 tensors).
+"""Fused multi-tensor SGD (one launch of sgd_multi_kernel for all 44 tensors, 58 with trunk conv biases).
 
 Semantics of ``torch.optim.SGD(params, lr, momentum, weight_decay=0)`` as the reference builds it
 (training.py:140, rebuilt at :252 on LR division => momentum buffers reset): v <- mu*v + g ; p <- p - lr*v.

@@ -29,9 +29,10 @@ N_BUCKETS = 5
 _LAST_LAYER_OF_BUCKET = {0: 10, 1: 8, 2: 6, 3: 2, 4: 0}
 
 
-def layer_of_param(i):
-    """index in UNet3D.ordered_parameters() (44 entries) -> layer index"""
-    return 14 if i >= 42 else i // 3
+def layer_of_param(i, stride=3):
+    """index in UNet3D.ordered_parameters() -> layer index; stride = UNet3D.trunk_stride() (3 trunk parameters per
+    layer, 4 with conv biases)"""
+    return 14 if i >= 14 * stride else i // stride
 
 
 class BucketedGradReducer(object):
@@ -47,10 +48,11 @@ class BucketedGradReducer(object):
             # weights or the averaged gradients are taken at different points and the replicas never agree
             broadcast_parameters(model, process_group)
         self.params = params
+        self.stride = model.trunk_stride()
         sizes = [0] * N_BUCKETS
         self.slot = []
         for i, p in enumerate(params):
-            b = _BUCKET_OF_LAYER[layer_of_param(i)]
+            b = _BUCKET_OF_LAYER[layer_of_param(i, self.stride)]
             n = (p.numel() + 3) // 4 * 4          # keep every view 16-byte aligned
             self.slot.append((b, sizes[b], p.numel()))
             sizes[b] += n
@@ -74,7 +76,7 @@ class BucketedGradReducer(object):
         """call before each backward: decides which layer closes each bucket given the requires_grad masks"""
         self._pending = []
         needs = [bool(p.requires_grad) for p in self.params]
-        active_layers = sorted({layer_of_param(i) for i, n in enumerate(needs) if n})
+        active_layers = sorted({layer_of_param(i, self.stride) for i, n in enumerate(needs) if n})
         self._close_at = {}
         for b in range(N_BUCKETS):
             layers = [l for l in active_layers if _BUCKET_OF_LAYER[l] == b]

@@ -32,6 +32,8 @@ _MODEL_DEFAULTS = (  # attribute, dict_model key, default, printed label
     ('interpolate', 'interpolate', True, 'Interpolate : '),
     ('final_sigmoid', 'final_sigmoid', False, 'Final Sigmoid : '),
     ('conv_layer_order', 'conv_layer_order', 'crg', 'Convolutional Layer Order : '),
+    # B200 extension: trunk convolutions with a bias (58-key checkpoints); a loaded checkpoint overrides it
+    ('conv_bias', 'conv_bias', False, 'Conv bias : '),
 )
 
 
@@ -313,6 +315,10 @@ class UnetPatternSulciLabelling(object):
         os.makedirs(op.join(self.working_path, 'models'), exist_ok=True)
         self.dict_model['model_file'] = self._model_path(name)
         self.dict_model['out_channels'] = len(self.sulci_side_list)
+        if self.model is not None and self.model.conv_bias:   # bias-free runs write the reference's keys only
+            self.dict_model['conv_bias'] = True
+        else:
+            self.dict_model.pop('conv_bias', None)
         params = {'dict_bck2': self.dict_bck2, 'dict_names': self.dict_names,
                   'sulci_side_list': self.sulci_side_list, 'dict_model': self.dict_model}
         if best_threshold is not None:
@@ -333,7 +339,8 @@ class UnetPatternSulciLabelling(object):
         self.model = UNet3D(dict_model['in_channels'], dict_model['out_channels'],
                             final_sigmoid=dict_model['final_sigmoid'], interpolate=dict_model['interpolate'],
                             conv_layer_order=dict_model['conv_layer_order'],
-                            init_channel_number=dict_model['init_channel_number'])
+                            init_channel_number=dict_model['init_channel_number'],
+                            conv_bias=dict_model.get('conv_bias', False))
         self.model.final_conv = make_head(dict_model['init_channel_number'], dict_model['out_channels'],
                                           dict_model['num_conv'])
         self.model.load_state_dict(torch.load(dict_model['model_file'], map_location='cpu'))

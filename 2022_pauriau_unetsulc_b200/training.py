@@ -35,7 +35,7 @@ class UnetTrainingSulciLabelling(UnetPatternSulciLabelling):
         print('Network initialization...')
         self.model = UNet3D(self.num_channel, len(self.sulci_side_list), final_sigmoid=self.final_sigmoid,
                             interpolate=self.interpolate, dropout=0., conv_layer_order=self.conv_layer_order,
-                            init_channel_number=self.num_filter)
+                            init_channel_number=self.num_filter, conv_bias=self.conv_bias)
         if self.num_conv > 1:
             # the reference reads an undefined self.dict_trained_model here (training.py:69); the filter count of
             # this model is the intended value

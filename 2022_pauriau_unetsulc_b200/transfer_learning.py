@@ -54,7 +54,7 @@ class UnetTransferSulciLabelling(UnetPatternSulciLabelling):
         print('Model_file: ', tm['model_file'])
         trained = UNet3D(tm['in_channels'], tm['out_channels'], final_sigmoid=tm['final_sigmoid'],
                          interpolate=tm['interpolate'], conv_layer_order=tm['conv_layer_order'],
-                         init_channel_number=tm['init_channel_number'])
+                         init_channel_number=tm['init_channel_number'], conv_bias=tm.get('conv_bias', False))
         if tm.get('num_conv', 1) > 1:
             trained.final_conv = make_head(tm['init_channel_number'], tm['out_channels'], tm['num_conv'])
         trained.load_state_dict(torch.load(tm['model_file'], map_location='cpu'))

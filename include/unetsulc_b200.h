@@ -64,6 +64,34 @@ int b2_relu_gn_bwd_acc(const long long* stat_acc, const void* dy, int lddy, int 
                        float* dbeta, void* workspace, long long workspace_bytes, const long long* dy_row_labels,
                        cudaStream_t stream);   /* dy_row_labels (may be NULL): see b2_head_ce_bstats */
 
+/* ---- convolutions with a bias (the 58-key checkpoint layout: double_conv.conv{1,2}.bias present) -----------------
+ * bias: fp32 [Cout] (8-byte aligned), added to the fp32 accumulator before ReLU, the bf16 rounding and the fused statistics (in
+ * 'crg' order the bias moves the ReLU threshold, GroupNorm does not absorb it).
+ * Tensor-core fprop: arguments of b2_conv3d_igemm; stat_acc (may be NULL) as b2_conv3d_igemm_stats; splitk_workspace
+ * (may be NULL, ignored with stat_acc or y_is_fp32) as b2_conv3d_igemm_splitk: the split partials stay bias-free, the
+ * reduction adds the bias once.  Every fprop path takes the bias (slab, implicit GEMM, fp32 output); launches that
+ * would take the opt-in CTA-pair kernel (B2_2CTA=1) run on the one-CTA kernel.                                     */
+int b2_conv3d_igemm_bias(const void* x, int ldx, int x_coff, const void* wpack, void* y, int ldy, int y_coff,
+                         int y_is_fp32, int N, int D, int H, int W, int Cin, int Cout, int relu, const float* bias,
+                         long long* stat_acc, void* splitk_workspace, long long splitk_workspace_bytes,
+                         cudaStream_t stream);
+/* first layer (Cin = 1) with a bias; stat_acc may be NULL, otherwise batch 1.  A voxel with no non-zero neighbour
+ * stores relu(bias).                                                                                               */
+int b2_conv3d_first_fwd_bias(const float* x, const float* w, const float* bias, void* y, int ldy, int y_coff, int N,
+                             int D, int H, int W, int Cout, int relu, long long* stat_acc, cudaStream_t stream);
+/* GroupNorm backward (the pass form b2_relu_gn_bwd and the accumulator form b2_relu_gn_bwd_acc, same arguments) that
+ * also produces the bias gradient dbias[c] = sum over samples and voxels of the stored bf16 dr[v, c].  The sums are
+ * fused into the apply pass and committed as fixed-point atomics into dbias_acc int64 [C][2] (zero before the call;
+ * bit-identical run to run); one more one-block launch writes dbias fp32 [C].  C <= 512.                            */
+int b2_relu_gn_bwd_dbias(const void* dy, int lddy, int dy_coff, const void* r, int N, long long V, int C, int G,
+                         const float* gamma, const float* mean_rstd, void* dr, float* dgamma, float* dbeta,
+                         void* workspace, long long workspace_bytes, int* counters, long long* dbias_acc, float* dbias,
+                         cudaStream_t stream);
+int b2_relu_gn_bwd_acc_dbias(const long long* stat_acc, const void* dy, int lddy, int dy_coff, const void* r,
+                             long long V, int C, int G, const float* gamma, const float* mean_rstd, void* dr,
+                             float* dgamma, float* dbeta, void* workspace, long long workspace_bytes,
+                             const long long* dy_row_labels, long long* dbias_acc, float* dbias, cudaStream_t stream);
+
 /* dW[co][ci][3][3][3] (fp32, PyTorch layout) = sum_v dY[v,co] * X[v+off,ci].  Cin: 16 or a multiple of 32; Cout: a
  * multiple of 32.  The workspace query returns -1 for any other shape.                                             */
 long long b2_conv3d_wgrad_workspace_bytes(int N, int D, int H, int W, int Cin, int Cout);
