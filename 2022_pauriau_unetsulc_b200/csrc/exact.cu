@@ -5,9 +5,12 @@
 // runs each 3x3x3 convolution on the SAME tcgen05 implicit-GEMM kernel with split operands ("bf16x3"):
 //     x = x_hi + x_lo (+ 2^-17 rel),  w = w_hi + w_lo     ->   x*w ~= x_hi*w_hi + x_lo*w_hi + x_hi*w_lo   (2^-16 rel)
 // realised as ONE convolution over 3*Cin input channels, [x_hi | x_lo | x_hi] against [w_hi | w_hi | w_lo], with fp32
-// accumulation in TMEM and an fp32 output.  The element-wise operators in between (ReLU is fused in the conv epilogue;
-// GroupNorm with fp64 statistics, MaxPool3d(2), trilinear upsample + concat, the 1x1x1 head + softmax at the skeleton
-// points) are the plain fp32 kernels below.  ~3x the convolution work of the bf16 path; inference only.
+// accumulation in TMEM and an fp32 output.  The first layer (Cin = 1) is split the same way into 32 channels,
+// [x_hi, x_hi, x_lo, 0...] against [w_hi, w_lo, w_hi, 0...], so any fp32 volume keeps its low half (for a binary
+// volume x_lo = 0 and the extra products are exact zeros).  The element-wise operators in between (ReLU is fused in
+// the conv epilogue; GroupNorm with fp64 statistics, MaxPool3d(2), trilinear upsample + concat, the 1x1x1 head +
+// softmax at the skeleton points) are the plain fp32 kernels below.  ~3x the convolution work of the bf16 path;
+// inference only.
 #include "common.h"
 #include <cuda_bf16.h>
 
@@ -40,15 +43,18 @@ exact_split3_kernel(const float* __restrict__ x, long long V, int C, int ldx, in
   }
 }
 
-// network input (binary, exact in bf16): out[v][0] = out[v][1] = x[v], channels 2..31 zero (pairs with [w_hi | w_lo | 0])
+// network input: out[v][0] = out[v][1] = hi(x), out[v][2] = lo(x), channels 3..31 zero (pairs with
+// [w_hi, w_lo, w_hi, 0...])
 __global__ void __launch_bounds__(256)
 exact_split_first_kernel(const float* __restrict__ x, long long V, __nv_bfloat16* __restrict__ out) {
   pdl_prologue();
   for (long long v = blockIdx.x * (long long)blockDim.x + threadIdx.x; v < V; v += (long long)gridDim.x * blockDim.x) {
-    const __nv_bfloat16 h = __float2bfloat16_rn(x[v]);
+    const float f = x[v];
+    const __nv_bfloat16 h = __float2bfloat16_rn(f);
+    const __nv_bfloat16 l = __float2bfloat16_rn(f - __bfloat162float(h));
     uint4* o = reinterpret_cast<uint4*>(out + v * 32);
     const uint32_t pair = (uint32_t)__bfloat16_as_ushort(h) | ((uint32_t)__bfloat16_as_ushort(h) << 16);
-    o[0] = make_uint4(pair, 0u, 0u, 0u);
+    o[0] = make_uint4(pair, (uint32_t)__bfloat16_as_ushort(l), 0u, 0u);
     o[1] = make_uint4(0u, 0u, 0u, 0u);
     o[2] = make_uint4(0u, 0u, 0u, 0u);
     o[3] = make_uint4(0u, 0u, 0u, 0u);
@@ -133,7 +139,7 @@ exact_gn_apply_kernel(const float* __restrict__ r, long long V, int C, const flo
   }
 }
 
-// MaxPool3d(2, 2, 0) on an fp32 NDHWC channel window
+// MaxPool3d(2, 2, 0) on an fp32 NDHWC channel window; a NaN anywhere in a cell makes the cell NaN (as torch.max_pool3d)
 __global__ void __launch_bounds__(256)
 exact_maxpool_kernel(const float* __restrict__ x, int N, int D, int H, int W, int C, int ldx, int xoff,
                      float* __restrict__ y) {
@@ -152,7 +158,8 @@ exact_maxpool_kernel(const float* __restrict__ x, int N, int D, int H, int W, in
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const long long v = (((long long)n * D + 2 * pd + (j >> 2)) * H + 2 * ph + ((j >> 1) & 1)) * W + 2 * pw + (j & 1);
-      m = fmaxf(m, x[v * ldx + xoff + c]);
+      const float f = x[v * ldx + xoff + c];
+      m = (f > m || f != f) ? f : m;
     }
     y[i] = m;
   }

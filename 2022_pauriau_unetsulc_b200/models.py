@@ -625,8 +625,9 @@ def _exact_methods():
                 lo = (w - hi).to(torch.bfloat16).float()
                 if l.cin == 1:
                     w3 = torch.zeros((l.cout, 32, 3, 3, 3), dtype=torch.float32, device=w.device)
-                    w3[:, 0] = hi[:, 0]
-                    w3[:, 1] = lo[:, 0]
+                    w3[:, 0] = hi[:, 0]     # x_hi * w_hi
+                    w3[:, 1] = lo[:, 0]     # x_hi * w_lo
+                    w3[:, 2] = hi[:, 0]     # x_lo * w_hi
                 else:
                     w3 = torch.cat([hi, hi, lo], dim=1).contiguous()
                 packs.append(ops.pack_conv_weights(w3, want_dgrad=False)[0])

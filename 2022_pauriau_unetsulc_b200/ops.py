@@ -798,7 +798,7 @@ def exact_split3(x, ld, off, C, D, H, W):
 
 
 def exact_split_first(x, D, H, W):
-    """network input fp32 [1, 1, D, H, W] -> ActView bf16 [1, D, H, W, 32] = [x, x, 0 ...]"""
+    """network input fp32 [1, 1, D, H, W] -> ActView bf16 [1, D, H, W, 32] = [hi, hi, lo, 0 ...]"""
     lib = _lib.load()
     out = ActView.alloc(1, D, H, W, 32, x.device)
     _lib.check(lib.b2_exact_split_first(_p(x), D * H * W, _p(out.buf), _s()), "b2_exact_split_first")
